@@ -1,80 +1,54 @@
 """Checkpoint / MPO interoperability with the reference's file formats (SURVEY 8(f4); pytdscf/simulator_cls.py:501-507,
-:577-589; pympo.utils.import_npz).  Fixtures made by tests/golden/make_golden_checkpoint.py with the unmodified reference:
-a reference-written ``wf_*.pkl`` and the energies of the reference continuing from it."""
+:577-589; pympo.utils.import_npz).  Fixture made by tests/golden/make_golden_checkpoint.py with the unmodified reference:
+its exciton state after 3 steps and the energies of the reference continuing from it."""
 import os
 import pickletools
-import shutil
 
 import numpy as np
 import pytest
 
-from tests.golden_io import GOLDEN_DIR, load_run
-
-REF_PKL = os.path.join(GOLDEN_DIR, "wf_ref_exciton_D6.pkl")
+from tests.golden_io import load_checkpoint, load_run, write_checkpoint
 
 
-def _golden():
-    return dict(np.load(os.path.join(GOLDEN_DIR, "checkpoint.npz")))
-
-
-def test_read_reference_pickle_without_the_reference_installed():
+def test_read_reference_pickle_without_the_reference_installed(tmp_path):
+    """The reference's state after 3 steps in its ``wf_*.pkl`` format (``tests.golden_io.write_checkpoint``; the reference
+    continued from such a file exactly as from its own dump) reads back without the reference installed."""
     import sys
 
     from pytdscf_b200.checkpoint import is_reference_pickle, read_reference_wavefunction
 
-    assert "pytdscf" not in sys.modules or not hasattr(sys.modules["pytdscf"], "Simulator")  # really not the reference
-    assert is_reference_pickle(REF_PKL)
-    d = read_reference_wavefunction(REF_PKL)
-    z = _golden()
-    assert d["gauges"] == [str(g) for g in z["gauges"]] == ["Psi", "B", "B", "B"]
-    for i, c in enumerate(d["cores"]):
-        assert c.dtype == np.complex128 and (c == z[f"core{i}"]).all()
-
-
-def test_written_file_has_the_reference_class_layout(tmp_path):
-    """Our writer emits the same class references and, per class, the same attribute names as the reference's own dump."""
-    from pytdscf_b200.checkpoint import _stub_unpickler, read_reference_wavefunction, write_reference_wavefunction
-
-    d = read_reference_wavefunction(REF_PKL)
-    path = write_reference_wavefunction(str(tmp_path / "wf_ours.pkl"), d["cores"], d["gauges"])
+    path = write_checkpoint(str(tmp_path / "wf_ck.pkl"))
     names = {arg for op, arg, _ in pickletools.genops(open(path, "rb").read()) if op.name == "SHORT_BINUNICODE" and isinstance(arg, str)}
     for module, cls in [("pytdscf.wavefunction", "WFunc"), ("pytdscf._mps_mpo", "MPSCoefMPO"), ("pytdscf._mps_cls", "LatticeInfo"),
                         ("pytdscf._site_cls", "SiteCoef"), ("pytdscf._spf_cls", "SPFCoef")]:
         assert module in names and cls in names
-    ours = _stub_unpickler(open(path, "rb")).load()
-    ref = _stub_unpickler(open(REF_PKL, "rb")).load()
-    assert set(vars(ours)) == {"ci_coef", "spf_coef", "ints_prim"} == set(vars(ref)) - {"ints_spf"}   # ints_spf: cache, rebuilt by WFunc(...)
-    assert set(vars(ours.ci_coef)) == set(vars(ref.ci_coef)) - {"matH_sweep"}   # cached operator: rebuilt by the reference
-    assert set(vars(ours.spf_coef)) == set(vars(ref.spf_coef))
-    assert set(vars(ours.ci_coef.lattice_info_states[0])) == set(vars(ref.ci_coef.lattice_info_states[0]))
-    assert vars(ours.ci_coef.lattice_info_states[0]) == vars(ref.ci_coef.lattice_info_states[0])
-    for a, b in zip(ours.ci_coef.superblock_states[0], ref.ci_coef.superblock_states[0], strict=True):
-        assert set(vars(a)) == set(vars(b)) and a.gauge == b.gauge and a.isite == b.isite and (np.asarray(a.data) == np.asarray(b.data)).all()
-    for a, b in zip(ours.spf_coef.data[0], ref.spf_coef.data[0], strict=True):
-        assert (np.asarray(a) == np.asarray(b)).all()
-    # and it round-trips through our own reader
-    back = read_reference_wavefunction(path)
-    assert back["gauges"] == d["gauges"] and all((x == y).all() for x, y in zip(back["cores"], d["cores"], strict=True))
-    z = _golden()
-    # tests/golden/make_golden_checkpoint.py: the reference restarted from OUR file reproduces its own continuation
+    assert "pytdscf" not in sys.modules or not hasattr(sys.modules["pytdscf"], "Simulator")  # really not the reference
+    assert is_reference_pickle(path)
+    d = read_reference_wavefunction(path)
+    z = load_checkpoint()
+    assert d["gauges"] == [str(g) for g in z["gauges"]] == ["Psi", "B", "B", "B"]
+    for i, c in enumerate(d["cores"]):
+        assert c.dtype == np.complex128 and (c == z[f"core{i}"]).all()
+    # tests/golden/make_golden_checkpoint.py: the reference restarted from such a file reproduces its own continuation
     assert (z["energies_restart_our_file"] == z["energies_restart_reference_file"]).all()
 
 
 def test_restart_from_a_reference_checkpoint_host_logic(tmp_path):
-    """Simulator(restart=True) picks up a reference-written wf_*.pkl and continues like the reference does (CPU host
-    logic with the oracle's kernels; the GPU version is in tests/test_gpu_propagation.py)."""
+    """Simulator(restart=True) picks up a wf_*.pkl in the reference's format (``tests.golden_io.write_checkpoint``) and
+    continues like the reference does (CPU host logic with the oracle's kernels; the GPU version is in
+    tests/test_gpu_propagation.py)."""
     import pytdscf_b200 as tb
     from oracle.oracle_engine import OracleEngine
     from tests.test_host_sweep_cpu import _build_model
 
     g = load_run("exciton_D6")
     os.chdir(tmp_path)
-    shutil.copy(REF_PKL, "wf_ck.pkl")
+    write_checkpoint("wf_ck.pkl")
     sim = tb.Simulator("ck", _build_model(g), backend="cuda", verbose=0)
     sim.eng = OracleEngine()
     ener, wf = sim.propagate(stepsize=0.1, maxstep=3, restart=True, loadfile_ext="", savefile_ext="_cont", autocorr=False,
                              norm=False, populations=False)
-    ref = _golden()["energies_restart_reference_file"]
+    ref = load_checkpoint()["energies_restart_reference_file"]
     got = [rec["energy"] for rec in sim.history]
     assert np.allclose(got, ref, rtol=0, atol=1e-13)
     # and hand the result back in the reference's format

@@ -293,19 +293,18 @@ def test_hermitise_mpdo_gpu(tag):
 
 
 def test_restart_from_reference_checkpoint_on_gpu(tmp_path):
-    """A ``wf_*.pkl`` written by the reference (dill dump of its WFunc) restarts on the GPU and continues with the
-    reference's own energies (tests/golden/make_golden_checkpoint.py), SURVEY 8(f4)."""
-    import shutil
-
+    """A ``wf_*.pkl`` in the reference's format (its WFunc layout) restarts on the GPU and continues with the reference's
+    own energies (tests/golden/make_golden_checkpoint.py), SURVEY 8(f4).  The file holds the reference's state after 3
+    steps (``tests.golden_io.write_checkpoint``), from which the reference itself continued exactly as from its own dump."""
     import pytdscf_b200 as tb
-    from tests.golden_io import GOLDEN_DIR
+    from tests.golden_io import load_checkpoint, write_checkpoint
 
     g = load_run("exciton_D6")
     os.chdir(tmp_path)
-    shutil.copy(os.path.join(GOLDEN_DIR, "wf_ref_exciton_D6.pkl"), "wf_ck.pkl")
+    write_checkpoint("wf_ck.pkl")
     sim = tb.Simulator("ck", build_model(g), backend="cuda", verbose=0)
     ener, wf = sim.propagate(stepsize=0.1, maxstep=3, restart=True, loadfile_ext="", savefile_ext="_cont", autocorr=False,
                              norm=False, populations=False)
-    ref = dict(np.load(os.path.join(GOLDEN_DIR, "checkpoint.npz")))["energies_restart_reference_file"]
+    ref = load_checkpoint()["energies_restart_reference_file"]
     for rec, e in zip(sim.history, ref, strict=True):
         assert abs(rec["energy"] - e) <= REL * abs(e)
