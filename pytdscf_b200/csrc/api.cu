@@ -119,7 +119,7 @@ int tdvp_create(int device, void* cuda_stream, tdvp_handle_t* out) {
       (e = cudaMalloc((void**)&h->gemm.sk_flags, sizeof(int) * (size_t)h->num_sms)) != cudaSuccess) { tdvp_destroy(h); return (int)e; }
   cudaMemsetAsync(h->gemm.sk_flags, 0, sizeof(int) * (size_t)h->num_sms, h->stream);
   int rc = 0;
-  if ((e = tdvp::zgemm_configure_device()) != cudaSuccess) rc = (int)e;
+  if ((e = tdvp::zgemm_configure_device(h->gemm)) != cudaSuccess) rc = (int)e;
   if (!rc) rc = tdvp::qr_configure(h);
   if (!rc) rc = tdvp::svd_configure(h);
   if (rc) { tdvp_destroy(h); return rc; }
@@ -278,9 +278,7 @@ int tdvp_zgemm(tdvp_handle_t h, int transA, int transB, int M, int N, int K, dou
   GemmDesc g = gemm_rowmajor(M, N, K, (const c128*)A, lda, transA != 0, transA == 2, (const c128*)B, ldb, transB != 0,
                              (c128*)C, ldc, c128{alpha_re, alpha_im}, c128{beta_re, beta_im});
   g.b_conj = transB == 2 ? 1 : 0;
-  cudaError_t e = zgemm_auto(g, h->gemm);
-  if (e != cudaSuccess) return cuda_fail(h, e, "zgemm_launch", __FILE__, __LINE__);
-  return 0;
+  return gemm(h, g);
 }
 
 }  // extern "C"

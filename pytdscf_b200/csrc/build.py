@@ -15,7 +15,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.dirname(HERE)
 SOURCES = ["api.cu", "zgemm.cu", "zgemm_tma.cu", "contract.cu", "krylov.cu", "qr.cu", "svd.cu"]
-HEADERS = ["common.cuh", "handle.cuh", "contract.cuh", os.path.join("..", "..", "include", "tdvp_b200.h")]
+HEADERS = ["common.cuh", "handle.cuh", "contract.cuh", "zgemm_plan.h", os.path.join("..", "..", "include", "tdvp_b200.h")]
 OUT = os.path.join(PKG, "libtdvp_b200.so")
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

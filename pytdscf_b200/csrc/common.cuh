@@ -59,7 +59,7 @@ struct GemmDesc {
   c128 alpha = {1.0, 0.0};
   c128 beta = {0.0, 0.0};
   const char* tag = "gemm";   // profiling label (static string)
-  // split-K (set by gemm_auto): blockIdx.z = batch * splitk + split; split s covers k in [s*k_chunk, (s+1)*k_chunk)
+  // split-K (set by zgemm_auto): blockIdx.z = batch * splitk + split; split s covers k in [s*k_chunk, (s+1)*k_chunk)
   // and writes its partial to C + s * c_split (then combined by the fixed-order reduction kernel).
   int splitk = 1;
   int k_chunk = 0;
@@ -86,19 +86,15 @@ struct GemmCtx {
   int* sk_flags = nullptr;
   int sk_slots = 0;
   mutable int sk_epoch = 0;
+  bool tma_encode = false;       // the driver offers cuTensorMapEncodeTiled (queried once per handle)
 };
 constexpr size_t STREAMK_TILE_ELEMS = 128 * 64;
-// Per-device kernel attributes (dynamic shared memory limits): called by tdvp_create for every new handle.
-cudaError_t zgemm_configure_device();
-// GEMM with automatic tile configuration and split-K for shapes that would leave most of the SMs idle (few output
-// tiles, long K): partial products go to ctx.scratch and are combined in fixed order by a second kernel, so results
-// stay deterministic.  Returns cudaGetLastError() of the launch.
+// Per-device kernel attributes (dynamic shared memory limits) and ctx.tma_encode: called by tdvp_create for every new handle.
+cudaError_t zgemm_configure_device(GemmCtx& ctx);
+// GEMM with automatic kernel, tile and split-K choice (plan_gemm in zgemm_plan.h); split-K partial products meet in a
+// thread-block cluster or in ctx.scratch and are combined in fixed order, so results stay deterministic.  Returns
+// cudaGetLastError() of the launch.
 cudaError_t zgemm_auto(const GemmDesc& d, const GemmCtx& ctx);
-// Persistent TMA-fed 128x64 kernel (zgemm_tma.cu).  zgemm_tma_try launches `d` (split-K fields resolved) when its operands
-// can be described by tensor maps and sets *used; otherwise nothing is launched and the caller uses the cp.async kernels.
-cudaError_t zgemm_tma_configure_device();
-cudaError_t zgemm_tma_try(const GemmDesc& d, const GemmCtx& ctx, bool* used);
-bool zgemm_tma_eligible(const GemmDesc& d);
 constexpr size_t SPLITK_SCRATCH_ELEMS = size_t(18) << 20;  // 288 MiB of partial products
 // Number of kernel launches issued through this library since load (bench.py's gpu_launches claim).
 void count_launch(unsigned long long n = 1);

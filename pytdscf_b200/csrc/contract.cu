@@ -130,12 +130,6 @@ int launch_check(Handle* h, const char* what) {
   return 0;
 }
 
-int gemm(Handle* h, const GemmDesc& g) {
-  cudaError_t e = zgemm_auto(g, h->gemm);
-  if (e != cudaSuccess) return cuda_fail(h, e, "zgemm_launch", __FILE__, __LINE__);
-  return 0;
-}
-
 int axpby2d(Handle* h, const c128* x, long long ldx, c128* y, long long ldy, long long rows, int cols, c128 alpha, c128 beta) {
   { ProfScope _ps(h->stream, "aux.axpby2d_kernel"); axpby2d_kernel<<<grid_for(rows * cols, 256), 256, 0, h->stream>>>(x, ldx, y, ldy, rows, cols, alpha, beta); }
   return launch_check(h, "axpby2d_kernel");
@@ -214,6 +208,12 @@ int stage2_diag(Handle* h, const c128* T1, const c128* Wd, c128* T2, int Dl, int
 }
 
 }  // namespace
+
+int gemm(Handle* h, const GemmDesc& g, const char* what) {
+  cudaError_t e = zgemm_auto(g, h->gemm);
+  if (e != cudaSuccess) return cuda_fail(h, e, what, __FILE__, __LINE__);
+  return 0;
+}
 
 size_t heff_ws_elems(const tdvp_heff_term* terms, int nterms, int Dl, int d, int Dr) {
   size_t need = 0;

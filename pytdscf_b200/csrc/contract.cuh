@@ -4,6 +4,9 @@
 
 namespace tdvp {
 
+// zgemm_auto on the handle's stream and GEMM context; a launch error is recorded on the handle as "CUDA error ... in <what>"
+int gemm(Handle* h, const GemmDesc& g, const char* what = "zgemm_launch");
+
 // workspace needs in complex128 elements (callers reserve before composing launches)
 size_t heff_ws_elems(const tdvp_heff_term* terms, int nterms, int Dl, int d, int Dr);
 size_t keff_ws_elems(const tdvp_keff_term* terms, int nterms, int Dl, int Dr);

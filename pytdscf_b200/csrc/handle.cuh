@@ -27,7 +27,7 @@ struct Handle {
   cudaEvent_t ev_main = nullptr, ev_side = nullptr;
   double* d_partial_side = nullptr;
   unsigned int* d_counter_side = nullptr;
-  GemmCtx gemm;                       // stream + scratch + overrides handed to every zgemm_auto call
+  GemmCtx gemm;                       // stream + scratch + overrides handed to every zgemm_auto call (gemm() in contract.cuh)
   // device limits queried once per handle (tdvp_create), never per process
   int num_sms = 148;
   int qr_max_cluster = 0;             // largest cluster the device co-schedules for k_qr_panel_cluster (0: none)

@@ -568,12 +568,6 @@ int lq(Handle* h, const char* what) {
   return 0;
 }
 
-int gemmq(Handle* h, const GemmDesc& g) {
-  cudaError_t e = zgemm_auto(g, h->gemm);
-  if (e != cudaSuccess) return cuda_fail(h, e, "zgemm_launch", __FILE__, __LINE__);
-  return 0;
-}
-
 }  // namespace
 
 constexpr int QR_MAX_SMS = 256;  // workspace bound for the per-CTA partials (B200: 148 SMs)
@@ -669,9 +663,9 @@ int qr_factor(Handle* h, c128* A, int m, int n, int lda, c128* Q, int ldq) {
       c128* Vp = Vall + (long long)j0 * lda + j0;
       c128* C = A + (long long)j0 * lda + j0 + jb;
       c128* T = Tall + (size_t)pnl * NB * NB;
-      TDVP_TRY(gemmq(h, vhc_desc(jb, nc, mp, Vp, lda, C, lda, W, "qr.VhC")));     // W = V^H C
-      TDVP_TRY(gemmq(h, tagged(gemm_rowmajor(jb, nc, jb, T, NB, true, true, W, nc, false, W2, nc, one, zero), "qr.TW")));      // W2 = T^H W
-      TDVP_TRY(gemmq(h, tagged(gemm_rowmajor(mp, nc, jb, Vp, lda, false, false, W2, nc, false, C, lda, mone, one), "qr.VW"))); // C -= V W2
+      TDVP_TRY(gemm(h, vhc_desc(jb, nc, mp, Vp, lda, C, lda, W, "qr.VhC")));     // W = V^H C
+      TDVP_TRY(gemm(h, tagged(gemm_rowmajor(jb, nc, jb, T, NB, true, true, W, nc, false, W2, nc, one, zero), "qr.TW")));      // W2 = T^H W
+      TDVP_TRY(gemm(h, tagged(gemm_rowmajor(mp, nc, jb, Vp, lda, false, false, W2, nc, false, C, lda, mone, one), "qr.VW"))); // C -= V W2
     }
   }
   // ---- form Q = H_1 ... H_k [I; 0]  (zungqr, blocked, backward) ----
@@ -685,9 +679,9 @@ int qr_factor(Handle* h, c128* A, int m, int n, int lda, c128* Q, int ldq) {
     c128* Vp = Vall + (long long)j0 * lda + j0;
     c128* C = Q + (long long)j0 * ldq + j0;
     c128* T = Tall + (size_t)pnl * NB * NB;
-    TDVP_TRY(gemmq(h, vhc_desc(jb, nc, mp, Vp, lda, C, ldq, W, "ungqr.VhC")));      // W = V^H C
-    TDVP_TRY(gemmq(h, tagged(gemm_rowmajor(jb, nc, jb, T, NB, false, false, W, nc, false, W2, nc, one, zero), "ungqr.TW")));     // W2 = T W
-    TDVP_TRY(gemmq(h, tagged(gemm_rowmajor(mp, nc, jb, Vp, lda, false, false, W2, nc, false, C, ldq, mone, one), "ungqr.VW")));  // C -= V W2
+    TDVP_TRY(gemm(h, vhc_desc(jb, nc, mp, Vp, lda, C, ldq, W, "ungqr.VhC")));      // W = V^H C
+    TDVP_TRY(gemm(h, tagged(gemm_rowmajor(jb, nc, jb, T, NB, false, false, W, nc, false, W2, nc, one, zero), "ungqr.TW")));     // W2 = T W
+    TDVP_TRY(gemm(h, tagged(gemm_rowmajor(mp, nc, jb, Vp, lda, false, false, W2, nc, false, C, ldq, mone, one), "ungqr.VW")));  // C -= V W2
   }
   return 0;
 }
@@ -726,10 +720,10 @@ int absorb_exec(Handle* h, int gauge, int Dl, int d, int Dr, int k, const c128* 
   TDVP_TRY(ws_reserve(h, 4096));
   if (gauge == TDVP_GAUGE_A) {
     // out(k, d*Dr) = sigma(k, Dl) . site(Dl, d*Dr)
-    return gemmq(h, tagged(gemm_rowmajor(k, d * Dr, Dl, sigma, Dl, false, false, site, (long long)d * Dr, false, out, (long long)d * Dr), "absorb"));
+    return gemm(h, tagged(gemm_rowmajor(k, d * Dr, Dl, sigma, Dl, false, false, site, (long long)d * Dr, false, out, (long long)d * Dr), "absorb"));
   } else if (gauge == TDVP_GAUGE_B) {
     // out(Dl*d, k) = site(Dl*d, Dr) . sigma(Dr, k)
-    return gemmq(h, tagged(gemm_rowmajor(Dl * d, k, Dr, site, Dr, false, false, sigma, k, false, out, k), "absorb"));
+    return gemm(h, tagged(gemm_rowmajor(Dl * d, k, Dr, site, Dr, false, false, sigma, k, false, out, k), "absorb"));
   }
   set_error(h, "absorb: bad gauge");
   return TDVP_ERR_ARG;

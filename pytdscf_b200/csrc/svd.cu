@@ -659,8 +659,7 @@ int tdvp_pinv(tdvp_handle_t hh, int m, int n, const tdvp_c128* X, double rcond, 
   GemmDesc g = gemm_rowmajor(n, m, n, Vh, n, true, true, U, n, true, (c128*)out, m);
   g.b_conj = 1;
   g.tag = "pinv";
-  cudaError_t e = zgemm_auto(g, h->gemm);
-  if (e != cudaSuccess) return cuda_fail(h, e, "zgemm(pinv)", __FILE__, __LINE__);
+  TDVP_TRY(gemm(h, g, "zgemm(pinv)"));
   TDVP_CUDA(h, cudaStreamSynchronize(h->stream));   // `inv` is a host temporary of the copy above
   return 0;
 }

@@ -16,10 +16,11 @@
 //    every fragment LDS.128 is bank-conflict free for both operand majors.
 //  * rows of A/C and columns of B may be two-level indices (GemmDesc) so contractions such as
 //    T2[a,i,t,s] = sum_{c,j} T1[a,c,j,s] W[c,i,j,t] run on their natural layouts (no transposes).
-//  * round 2: this file keeps the cp.async kernels (three tile geometries), the launch choice (choose(): tile, split-K
-//    factor) and the two split-K forms -- scratch + fixed-order reduction kernel, and, for the small tiles, a thread-block
-//    cluster per output tile that reduces the partial tiles through distributed shared memory.  The 128x64 work of the
-//    D >= 256 regime runs in the persistent TMA-fed kernel of zgemm_tma.cu whenever tensor maps can describe the operands.
+//  * round 2: this file keeps the cp.async kernels (three tile geometries), zgemm_auto and the two split-K forms --
+//    scratch + fixed-order reduction kernel, and, for the small tiles, a thread-block cluster per output tile that reduces
+//    the partial tiles through distributed shared memory.  The 128x64 work of the D >= 256 regime runs in the persistent
+//    TMA-fed kernel of zgemm_tma.cu whenever tensor maps can describe the operands.  Which kernel, tile, split-K factor and
+//    reduction a GEMM gets is decided by plan_gemm (zgemm_plan.h); zgemm_auto only executes the plan.
 #include <cooperative_groups.h>
 
 #include <atomic>
@@ -29,7 +30,7 @@
 #include <string>
 #include <vector>
 
-#include "common.cuh"
+#include "zgemm_plan.h"
 
 namespace tdvp {
 
@@ -456,93 +457,6 @@ cudaError_t launch_cfg(const GemmDesc& d, cudaStream_t stream) {
   return cudaGetLastError();
 }
 
-inline long long tiles_of(const GemmDesc& d, int bm, int bn) {
-  return (long long)((d.M + bm - 1) / bm) * ((d.N + bn - 1) / bn) * d.batch;
-}
-
-// Cost model of one launch (measured constants, profiles/r1_zgemm_cfg_sweep.json): a CTA tile of configuration c costs
-// `lone` seconds per unit of k when it has an SM to itself and `full` when `cps` of them share the SM; K0 = prologue +
-// epilogue in units of k.  time = waves * (k_chunk + K0) * per_k  (+ the fixed-order reduction for split-K).
-struct CfgModel { int id, bm, bn, bk, cps, min_chunk; double lone, full, K0, bias; };
-constexpr CfgModel MODELS[4] = {
-    {4, 128, 64, 16, 1, 128, 0.2606e-6, 0.2606e-6, 40.0, 1.00},  // tma: persistent big tile (7.70 ms on 8192x4096x1024, 0.231 ms on
-                                                                 // 1280x2560x256: profiles/r2_zgemm_shapes_tma.jsonl); replaces "big"
-                                                                 // whenever tensor maps can describe the operands
-    {1, 128, 64, 16, 1, 128, 0.282e-6, 0.282e-6, 32.0, 1.00},  // big   (8.33 ms / 28 waves / 1056 k on 8192x4096x1024)
-    {2, 64, 32, 8, 4, 64, 0.075e-6, 0.30e-6, 24.0, 1.00},      // small (only when forced: never the best in the sweep)
-    {3, 32, 32, 8, 4, 32, 0.040e-6, 0.140e-6, 16.0, 1.00},     // tiny  (832 us / 10.9 waves / 528 k on 1536x4096x512)
-};
-struct Choice { int cfg = 1, S = 1, chunk = 0; double t = 1e30; };
-
-// split-K through a thread-block cluster (GemmDesc::cluster_sk): tiny and small tiles, clusters of up to 16 CTAs (the
-// non-portable size sm_100 offers; allowed per kernel in configure_cfg), one batch; force_cstream = 1 (a test override) keeps the scratch + reduction-kernel path reachable for the tests
-inline bool cluster_splitk_ok(int cfg, int S, const GemmDesc& d, const GemmCtx& ctx) {
-  return (cfg == 2 || cfg == 3) && S >= 2 && S <= 16 && d.batch == 1 && ctx.force_cstream != 1;
-}
-
-inline Choice choose(const GemmDesc& d, const GemmCtx& ctx) {
-  Choice best;
-  const bool allow_split = ctx.scratch != nullptr && ctx.force_splitk != 1;
-  const size_t scratch_elems = ctx.scratch_elems;
-  // force_cfg 4 (tma) shares the big tile's geometry: the split-K factor is chosen as for the forced big configuration
-  const int forced = ctx.force_cfg >= 4 ? 1 : (ctx.force_cfg >= 1 && ctx.force_cfg <= 3 ? ctx.force_cfg : 0);
-  const double bw = 5.0e12;
-  // >= 8 full waves of big tiles with a long K: wave quantisation is < 6 % and the big tiles need the least L2 traffic
-  // per flop (short-K GEMMs such as H_eff stage 2 are prologue-bound and keep the free choice)
-  const bool large = tiles_of(d, 128, 64) >= 8 * 148 && d.K >= 512;
-  const bool tma_ok = (ctx.force_cfg == 0 || ctx.force_cfg >= 4) && zgemm_tma_eligible(d);
-  for (const CfgModel& m : MODELS) {
-    if (m.id == 4 ? !tma_ok : (m.id == 1 && tma_ok)) continue;           // the TMA kernel stands in for the big tile
-    const int mid = m.id == 4 ? 1 : m.id;                                 // ... and shares its geometry / forcing rules
-    if (forced ? forced != mid : (mid == 2 || (large && mid != 1))) continue;
-    const long long tiles = tiles_of(d, m.bm, m.bn);
-    const int slots = 148 * m.cps;
-    int max_s = 1;
-    if (allow_split && d.batch == 1 && d.K >= 2 * m.min_chunk && (tiles < 8 * 148 || ctx.force_splitk >= 2)) {
-      max_s = d.K / m.min_chunk < 16 ? d.K / m.min_chunk : 16;
-    }
-    // tdvp_set_gemm_config(splitk = S >= 2): exactly that factor when the shape allows it (tests of the split-K path)
-    const int min_s = (ctx.force_splitk >= 2 && max_s >= 2) ? (ctx.force_splitk < max_s ? ctx.force_splitk : max_s) : 1;
-    if (min_s > 1) max_s = min_s;
-    for (int S = min_s; S <= max_s; ++S) {
-      int chunk = (d.K + S - 1) / S;
-      chunk = (chunk + m.bk - 1) / m.bk * m.bk;
-      if ((d.K + chunk - 1) / chunk != S) continue;
-      if (S > 1 && (size_t)S * d.M * d.N > scratch_elems) break;
-      const long long units = tiles * S;
-      double per_k = m.full;
-      if (units <= 148) per_k = m.lone;
-      else if (units < slots) per_k = m.lone * (double)((units + 147) / 148);
-      // big tiles run in lock-step waves (1 CTA per SM); the 4-per-SM tiny CTAs are scheduled dynamically, which the
-      // sweep fits as fractional waves + half a wave of tail
-      double waves = (double)((units + slots - 1) / slots);
-      if (m.id == 3 && units >= slots) waves = (double)units / slots + 0.5;
-      // the TMA kernel cuts the tiles x k-tiles space evenly over the SMs (stream-K): fractional waves + the fix-up (with
-      // half..all as many tiles as SMs a tile is shared by two CTAs, one ~4 us hand-over)
-      double sk_extra = 0.0;
-      if (m.id == 4 && S == 1 && ctx.force_cfg != 5 && ctx.sk_ws) {
-        if (units >= slots && d.K >= 256) waves = (double)units / slots + 0.1;
-        else if (2 * units >= slots && d.K >= 512) { waves = (double)units / slots; sk_extra = 4.0e-6; }
-      }
-      double t = waves * (chunk + m.K0) * per_k * m.bias + sk_extra;
-      // split-K pays a second launch; in the launch-bound small-D regime that launch costs a full ~9 us slot of the stream
-      // (r2 c2 profile: 2300 reduction launches per step), elsewhere ~4 us
-      // -- unless the S CTAs of a tile can be a cluster (tiny / small tiles, S <= 8): then the partials meet in
-      // distributed shared memory inside the same launch (two cluster barriers, ~2 us)
-      if (S > 1 && cluster_splitk_ok(mid, S, d, ctx)) t += 2.0e-6;
-      else if (S > 1) t += (double)(S + 2) * d.M * d.N * 16.0 / bw + ((double)d.M * d.N * d.K < 5.0e7 ? 9.0e-6 : 4.0e-6);
-      if (t < best.t * (S > 1 && best.cfg == mid ? 0.97 : 1.0)) { best.t = t; best.cfg = mid; best.S = S; best.chunk = chunk; }
-    }
-  }
-  return best;
-}
-
-inline cudaError_t launch_by_cfg(int cfg, const GemmDesc& d, cudaStream_t stream) {
-  if (cfg == 3) return launch_cfg<TinyCfg>(d, stream);
-  if (cfg == 2) return launch_cfg<SmallCfg>(d, stream);
-  return launch_cfg<BigCfg>(d, stream);
-}
-
 }  // namespace
 
 namespace {
@@ -566,9 +480,15 @@ __global__ void k_splitk_reduce(const c128* __restrict__ P, int S, int M, int N,
 }
 }  // namespace
 
-cudaError_t zgemm_configure_device() {
+cudaError_t zgemm_dmma_launch(int kernel, const GemmDesc& d, cudaStream_t stream) {
+  if (kernel == GEMM_TINY) return launch_cfg<TinyCfg>(d, stream);
+  if (kernel == GEMM_SMALL) return launch_cfg<SmallCfg>(d, stream);
+  return launch_cfg<BigCfg>(d, stream);
+}
+
+cudaError_t zgemm_configure_device(GemmCtx& ctx) {
   cudaError_t e;
-  if ((e = zgemm_tma_configure_device())) return e;
+  if ((e = zgemm_tma_configure_device(ctx))) return e;
   if ((e = configure_cfg<BigCfg>())) return e;
   if ((e = configure_cfg<SmallCfg>())) return e;
   return configure_cfg<TinyCfg>();
@@ -576,51 +496,32 @@ cudaError_t zgemm_configure_device() {
 
 cudaError_t zgemm_auto(const GemmDesc& d, const GemmCtx& ctx) {
   if (d.M <= 0 || d.N <= 0 || d.batch <= 0) return cudaSuccess;
-  cudaStream_t stream = ctx.stream;
-  c128* scratch = ctx.scratch;
-  // wave-aware choice of the tile configuration AND the split-K factor (see choose())
-  const Choice ch = choose(d, ctx);
-  const int S = ch.S, chunk = ch.chunk;
-  // the big-tile work goes to the persistent TMA kernel whenever tensor maps can describe the operands
-  const bool want_tma = ctx.force_cfg >= 4 || (ctx.force_cfg == 0 && ch.cfg == 1);
-  auto launch = [&](const GemmDesc& g) -> cudaError_t {
-    if (want_tma) {
-      bool used = false;
-      cudaError_t e = zgemm_tma_try(g, ctx, &used);
-      if (used || e != cudaSuccess) return e;
-    }
-    return launch_by_cfg(ch.cfg, g, stream);
-  };
-  if (S < 2) {
-    GemmDesc g1 = d;
-    // outputs larger than half of L2 are written with evict-first stores
-    g1.c_stream = ctx.force_cstream ? (ctx.force_cstream == 1) : ((double)d.M * d.N * d.batch * 16.0 > 64.0e6);
-    return launch(g1);
-  }
-  if (!want_tma && cluster_splitk_ok(ch.cfg, S, d, ctx)) {
-    GemmDesc g = d;
-    g.splitk = S;
-    g.k_chunk = chunk;
+  const GemmPlan pl = plan_gemm(d, ctx);
+  GemmDesc g = d;
+  g.c_stream = pl.c_stream;
+  if (pl.reduce == REDUCE_CLUSTER) {
+    g.splitk = pl.S;
+    g.k_chunk = pl.k_chunk;
     g.c_split = 0;
     g.cluster_sk = 1;
-    return launch_by_cfg(ch.cfg, g, stream);
+  } else if (pl.reduce == REDUCE_SCRATCH) {
+    g.C = ctx.scratch;
+    g.c_m_inner = 1; g.c_m1 = d.N; g.c_m0 = 0; g.c_n = 1; g.c_batch = 0;
+    g.alpha = {1.0, 0.0};
+    g.beta = {0.0, 0.0};
+    g.splitk = pl.S;
+    g.k_chunk = pl.k_chunk;
+    g.c_split = (long long)d.M * d.N;
   }
-  GemmDesc g = d;
-  g.C = scratch;
-  g.c_m_inner = 1; g.c_m1 = d.N; g.c_m0 = 0; g.c_n = 1; g.c_batch = 0;
-  g.alpha = {1.0, 0.0};
-  g.beta = {0.0, 0.0};
-  g.splitk = S;
-  g.k_chunk = chunk;
-  g.c_split = (long long)d.M * d.N;
-  cudaError_t e = launch(g);
-  if (e != cudaSuccess) return e;
+  const bool tma = pl.kernel == GEMM_TMA_WIDE || pl.kernel == GEMM_TMA_TALL;
+  cudaError_t e = tma ? zgemm_tma_launch(g, pl, ctx) : zgemm_dmma_launch(pl.kernel, g, ctx.stream);
+  if (e != cudaSuccess || pl.reduce != REDUCE_SCRATCH) return e;
   const long long tot = (long long)d.M * d.N;
   int blocks = (int)((tot + 255) / 256);
   if (blocks > 148 * 8) blocks = 148 * 8;
   {
-    ProfScope scope(stream, "aux.k_splitk_reduce");
-    k_splitk_reduce<<<blocks, 256, 0, stream>>>(scratch, S, d.M, d.N, (long long)d.M * d.N, d);
+    ProfScope scope(ctx.stream, "aux.k_splitk_reduce");
+    k_splitk_reduce<<<blocks, 256, 0, ctx.stream>>>(ctx.scratch, pl.S, d.M, d.N, (long long)d.M * d.N, d);
   }
   count_launch();
   return cudaGetLastError();

@@ -16,71 +16,25 @@
 //    k = 4 (q >> 1) + t, is chosen so that every LDS phase hits 8 distinct 16-byte bank groups for k-contiguous AND
 //    row-contiguous operands (bank arithmetic in DESIGN.md 4.1b).
 // Shapes the tensor maps cannot express (batched, rows not a multiple of 8 on a row-contiguous operand, two-level row
-// indices that do not tile by 128 / 64) fall back to the cp.async kernels of zgemm.cu.
+// indices that do not tile by 128 / 64) run on the cp.async kernels of zgemm.cu (plan_gemm, zgemm_plan.h).
 #include <cuda.h>
 #include <cudaTypedefs.h>
 
 #include <mutex>
 
-#include "common.cuh"
+#include "zgemm_plan.h"
 
 namespace tdvp {
 
 namespace {
 
-constexpr int BK = 16;
+constexpr int BK = TMA_BK;
 constexpr int CONSUMER_WARPS = 8;
-// Two tile geometries, both 8 consumer warps of 32 x 32: 4 x 2 warps (CTA tile 128 x 64, 4 stages) for the bulk of the work and
-// 8 x 1 warps (256 x 32, 3 stages) for GEMMs whose N is at most 32 (H_eff stage 2 at d w <= 32: with a 64-wide tile half of
-// every B fragment would be zero padding).
-template <int WMW_, int WNW_, int STAGES_>
-struct TmaCfg {
-  static constexpr int WMW = WMW_, WNW = WNW_, STAGES = STAGES_;
-  static constexpr int BM = 32 * WMW, BN = 32 * WNW;
-  static constexpr int SLAB_A = BM * 128, SLAB_B = BN * 128;          // bytes of one 8-k slab of the A / B tile
-  static constexpr int STAGE_BYTES = 2 * (SLAB_A + SLAB_B);            // two slabs (BK = 16) of both operands
-  static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024 + 256;  // + alignment slack + barriers
-  static_assert(WMW * WNW == CONSUMER_WARPS, "8 consumer warps");
-};
-using WideCfg = TmaCfg<4, 2, 4>;     // 128 x 64, 4 x 48 KiB
-using TallCfg = TmaCfg<8, 1, 3>;     // 256 x 32, 3 x 72 KiB
 // Registers are allocated per warpgroup (4 warps): 2 consumer warpgroups + 1 producer warpgroup (one working lane).  The
 // launch gives every thread 168 registers (65536 / 384); the producer group then shrinks to 40 and the consumers grow
 // to 232 with setmaxnreg, as warp-specialised Hopper / Blackwell GEMMs do.
 constexpr int THREADS = 32 * (CONSUMER_WARPS + 4);
 constexpr int PRODUCER_REGS = 40, CONSUMER_REGS = 232;
-constexpr unsigned BIG_INNER = 1u << 30;                      // "plain" operand: a single row level
-
-struct TmaSide {
-  unsigned inner;      // rows per step of the outer row index (BIG_INNER: plain matrix)
-  short small_inner;   // inner < tile rows: the box spans several outer steps
-  short swapped;       // k-contiguous operand whose two row levels are listed (outer, inner) in the tensor map so that its
-                       // strides ascend (the box has extent 1 in the outer level, the shared-memory image is the same)
-};
-
-struct TmaParams {
-  int M, N, K, tiles_m, tiles_n, splitk, k_chunk;
-  int group_m;         // M-tiles walked per N-tile before moving on: the A rows of a group stay in L2 while B streams
-  TmaSide a, b;
-  unsigned a_conj, b_conj;
-  c128* C;
-  int c_m_inner;
-  long long c_m1, c_m0, c_n, c_split;
-  c128 alpha, beta;
-  int c_stream;
-  // stream-K (splitk == 1, at least one tile per CTA): the tiles x k-tiles iteration space is cut into gridDim.x equal
-  // contiguous ranges; a tile that straddles two ranges is finished by the second CTA from the first one's partial sums
-  int streamk;         // 0: whole tiles round-robin (and split-K work items)
-  int sk_tiles;        // stream-K: tiles [0, sk_tiles) are cut evenly over the CTAs, the rest are whole waves
-  int epoch;           // value the head writer stores into sk_flags[cta] (grows with every launch: no reset needed)
-  int* sk_flags;       // one per CTA
-  c128* sk_ws;         // one BM x BN accumulator image per CTA, in fragment order
-};
-
-struct Seg {
-  int tm, tn, split, kt0, kt1, role;   // role 0: whole tile (or split-K item), 1: head part -> publish, 2: tail part -> finish,
-                                       // 3: middle part (ranges shorter than a tile) -> add the predecessor's sums, publish
-};
 
 __device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(unsigned bar, unsigned count) {
@@ -123,78 +77,6 @@ __device__ __forceinline__ void dmma(double& c0, double& c1, double a, double b)
   asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n" : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
 }
 
-// Work item w -> (tile_m, tile_n, split): splits outermost, then the grouped rasterisation of zgemm_dmma_kernel (group_m
-// M-tiles per N-tile), so the CTAs of one persistent "wave" (consecutive w) share A rows / B columns in L2.
-__device__ __forceinline__ void decode_work(const TmaParams& p, int w, int& tm, int& tn, int& split) {
-  const int GROUP_M = p.group_m;
-  const int per_split = p.tiles_m * p.tiles_n;
-  split = w / per_split;
-  const int pid = w - split * per_split;
-  const int in_group = GROUP_M * p.tiles_n;
-  const int first_m = (pid / in_group) * GROUP_M;
-  const int gsz = (p.tiles_m - first_m) < GROUP_M ? (p.tiles_m - first_m) : GROUP_M;
-  tm = first_m + (pid % in_group) % gsz;
-  tn = (pid % in_group) / gsz;
-}
-
-// Number of segments of this CTA and the si-th of them.  Stream-K is applied to the FIRST p.sk_tiles tiles of the raster only
-// (between one and two waves' worth, or everything when there are fewer tiles than that): their tiles x k-tiles space is cut
-// into gridDim.x equal contiguous ranges.  The remaining tiles are whole waves and keep the strided persistent order
-// (tile = sk_tiles + w * grid + cta), in which the CTAs of a wave share A rows / B columns in L2 -- cutting the WHOLE raster
-// into per-CTA ranges would put every CTA into a different region of the matrix at any moment and defeat that reuse
-// (measured: 11 GB of DRAM reads instead of 0.5 GB on 8192 x 4096 x 1024).
-// Order inside the stream-K part: the trailing partial tile (the HEAD part of a tile the next CTA finishes) first, then the
-// whole tiles, the leading partial tile (TAIL part, finished here from the previous CTA's partial) last -- so a finisher
-// never waits for work its neighbour has not started with.
-__device__ __forceinline__ int sk_seg_count(const TmaParams& p, int KT) {
-  const long long I = (long long)p.sk_tiles * KT;
-  const long long a = I * blockIdx.x / gridDim.x, b = I * (blockIdx.x + 1) / gridDim.x;
-  if (b <= a) return 0;
-  const int first = (int)(a / KT), last = (int)((b - 1) / KT);
-  return last - first + 1;       // lead (partial or whole) + middle tiles + trail (partial or whole)
-}
-__device__ __forceinline__ int seg_count(const TmaParams& p, int KT) {
-  const int total = p.tiles_m * p.tiles_n * p.splitk;
-  if (!p.streamk) return (int)blockIdx.x < total ? (total - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x : 0;
-  const int rest = total - p.sk_tiles;    // a multiple of gridDim.x
-  return sk_seg_count(p, KT) + rest / (int)gridDim.x;
-}
-
-__device__ __forceinline__ Seg get_seg(const TmaParams& p, int si, int KT) {
-  Seg sg;
-  if (!p.streamk) {
-    const int w = blockIdx.x + si * gridDim.x;
-    decode_work(p, w, sg.tm, sg.tn, sg.split);
-    const int k_begin = sg.split * p.k_chunk;
-    const int k_end = (p.splitk > 1 && k_begin + p.k_chunk < p.K) ? k_begin + p.k_chunk : p.K;
-    sg.kt0 = 0;
-    sg.kt1 = (k_end - k_begin + BK - 1) / BK;
-    sg.role = 0;
-    return sg;
-  }
-  const int n = sk_seg_count(p, KT);
-  if (si >= n) {                             // whole waves after the stream-K part
-    decode_work(p, p.sk_tiles + (si - n) * (int)gridDim.x + (int)blockIdx.x, sg.tm, sg.tn, sg.split);
-    sg.kt0 = 0; sg.kt1 = KT; sg.role = 0;
-    return sg;
-  }
-  const long long I = (long long)p.sk_tiles * KT;
-  const long long a = I * blockIdx.x / gridDim.x, b = I * (blockIdx.x + 1) / gridDim.x;
-  const int first = (int)(a / KT), a_off = (int)(a % KT), last = (int)((b - 1) / KT), b_off = (int)(b - (long long)last * KT);
-  int tile;
-  if (first == last) {                       // the whole range lies in one tile
-    tile = first; sg.kt0 = a_off; sg.kt1 = b_off;
-    sg.role = (a_off == 0 && b_off == KT) ? 0 : (a_off == 0 ? 1 : (b_off == KT ? 2 : 3));
-  } else {
-    // order: [trail, middle..., lead]
-    if (si == 0) { tile = last; sg.kt0 = 0; sg.kt1 = b_off; sg.role = b_off == KT ? 0 : 1; }
-    else if (si == n - 1) { tile = first; sg.kt0 = a_off; sg.kt1 = KT; sg.role = a_off == 0 ? 0 : 2; }
-    else { tile = first + si; sg.kt0 = 0; sg.kt1 = KT; sg.role = 0; }
-  }
-  decode_work(p, tile, sg.tm, sg.tn, sg.split);
-  return sg;
-}
-
 template <bool KMAJOR>
 __device__ __forceinline__ void issue_box(unsigned dst, const CUtensorMap* map, unsigned bar, const TmaSide& s, int row0, int k0) {
   const int lo = s.small_inner ? 0 : (int)((unsigned)row0 % s.inner);
@@ -228,7 +110,7 @@ __global__ void __launch_bounds__(THREADS, 1)
   }
   __syncthreads();
   const int KT_full = (p.K + BK - 1) / BK;
-  const int nseg = seg_count(p, KT_full);
+  const int nseg = seg_count(p, KT_full, blockIdx.x, gridDim.x);
 
   if (warp >= CONSUMER_WARPS) {
     // ================= producer: one lane walks the same work list and keeps the ring full =================
@@ -239,7 +121,7 @@ __global__ void __launch_bounds__(THREADS, 1)
     int stage = 0;
     unsigned phase = 0;
     for (int si = 0; si < nseg; ++si) {
-      const Seg sg = get_seg(p, si, KT_full);
+      const Seg sg = get_seg(p, si, KT_full, blockIdx.x, gridDim.x);
       const int tm = sg.tm, tn = sg.tn;
       const int k_begin = sg.split * p.k_chunk;
       for (int kt = sg.kt0; kt < sg.kt1; ++kt) {
@@ -307,7 +189,7 @@ __global__ void __launch_bounds__(THREADS, 1)
   const c128 alpha = p.alpha, beta = p.beta;
   const bool use_beta = (beta.x != 0.0) || (beta.y != 0.0);
   for (int si = 0; si < nseg; ++si) {
-    const Seg sg = get_seg(p, si, KT_full);
+    const Seg sg = get_seg(p, si, KT_full, blockIdx.x, gridDim.x);
     const int tm = sg.tm, tn = sg.tn, split = sg.split;
     const int KT = sg.kt1 - sg.kt0;
 #pragma unroll
@@ -424,104 +306,11 @@ PFN_cuTensorMapEncodeTiled encode_fn() {
   return fn;
 }
 
-inline cuuint64_t clamp_stride(unsigned long long s) {
-  const unsigned long long cap = (1ull << 40) - 16;
-  return s < 16 ? 16 : (s > cap ? cap : s);
-}
-
-// One operand with `rows` rows (two-level: row = r1 * inner + r0) and K columns, element (row, k) at
-// ptr + r1 * s1 + r0 * s0 + k * sk (complex128 units).  R = tile rows (128 for A, 64 for B).  Returns false when the
-// operand cannot be described (the caller then uses the cp.async kernel).
-struct SidePlan {
-  cuuint64_t dims[4], strides[3];
-  cuuint32_t box[4];
-};
-
-bool plan_side(SidePlan* pl, TmaSide* side, bool* kmajor, const c128* ptr, long long rows, int K, int inner, long long s1,
-               long long s0, long long sk, int R) {
-  cuuint64_t* dims = pl->dims;
-  cuuint64_t* strides = pl->strides;
-  cuuint32_t* box = pl->box;
-  if (rows <= 0 || K < BK) return false;
-  if ((reinterpret_cast<uintptr_t>(ptr) & 15u) != 0) return false;
-  if (inner <= 0) return false;
-  const bool two = inner > 1 && inner < rows;
-  if (!two) {           // single row level: fold it into (inner = 1, s1)
-    if (inner > 1) { s1 = s0; }   // rows <= inner: only the r0 level is walked
-    inner = 1;
-  } else if (rows % inner != 0) {
-    return false;
-  }
-  if (sk == 1) {
-    *kmajor = true;
-    if (!two) {
-      dims[0] = 2ull * K; dims[1] = (cuuint64_t)rows; dims[2] = 1; dims[3] = 1;
-      strides[0] = clamp_stride(16ull * s1);
-      strides[1] = clamp_stride(strides[0] * (unsigned long long)rows);
-      strides[2] = strides[1];
-      box[0] = 16; box[1] = R; box[2] = 1; box[3] = 1;
-      side->inner = BIG_INNER; side->small_inner = 0; side->swapped = 0;
-      if (s1 < 1) return false;
-    } else {
-      if (inner % R != 0 && R % inner != 0) return false;
-      if (s0 < 1 || s1 < 1) return false;
-      const long long n1 = rows / inner;
-      const bool small = inner < R;
-      const bool swap = !small && s0 > s1;
-      dims[0] = 2ull * K; dims[3] = 1;
-      if (!swap) {
-        dims[1] = (cuuint64_t)inner; dims[2] = (cuuint64_t)n1;
-        strides[0] = clamp_stride(16ull * s0);
-        strides[1] = clamp_stride(16ull * s1);
-        strides[2] = clamp_stride(strides[1] * (unsigned long long)n1);
-        box[0] = 16; box[1] = small ? inner : R; box[2] = small ? R / inner : 1; box[3] = 1;
-      } else {
-        dims[1] = (cuuint64_t)n1; dims[2] = (cuuint64_t)inner;
-        strides[0] = clamp_stride(16ull * s1);
-        strides[1] = clamp_stride(16ull * s0);
-        strides[2] = clamp_stride(strides[1] * (unsigned long long)inner);
-        box[0] = 16; box[1] = 1; box[2] = R; box[3] = 1;
-      }
-      side->inner = (unsigned)inner; side->small_inner = small ? 1 : 0; side->swapped = swap ? 1 : 0;
-    }
-  } else {
-    *kmajor = false;
-    if (sk < 8) return false;        // k stride must cover the 8-row (128-byte) inner box
-    if (!two) {
-      if (s1 != 1 || rows % 8 != 0) return false;
-      dims[0] = 16; dims[1] = (cuuint64_t)K; dims[2] = (cuuint64_t)(rows / 8); dims[3] = 1;
-      strides[0] = clamp_stride(16ull * sk);
-      strides[1] = 128;
-      strides[2] = clamp_stride(128ull * (unsigned long long)(rows / 8));
-      box[0] = 16; box[1] = 8; box[2] = R / 8; box[3] = 1;
-      side->inner = BIG_INNER; side->small_inner = 0; side->swapped = 0;
-    } else {
-      if (s0 != 1 || inner % 8 != 0) return false;
-      if (inner % R != 0 && R % inner != 0) return false;
-      dims[0] = 16; dims[1] = (cuuint64_t)K; dims[2] = (cuuint64_t)(inner / 8); dims[3] = (cuuint64_t)(rows / inner);
-      strides[0] = clamp_stride(16ull * sk);
-      strides[1] = 128;
-      strides[2] = clamp_stride(16ull * s1);
-      const bool small = inner < R;
-      box[0] = 16; box[1] = 8; box[2] = (small ? inner : R) / 8; box[3] = small ? R / inner : 1;
-      side->inner = (unsigned)inner; side->small_inner = small ? 1 : 0; side->swapped = 0;
-      if (s1 < 1) return false;
-    }
-  }
-  for (int i = 0; i < 3; ++i)
-    if (strides[i] % 16 != 0) return false;
-  return true;
-}
-
-bool make_side(CUtensorMap* map, TmaSide* side, bool* kmajor, const c128* ptr, long long rows, int K, int inner, long long s1,
-               long long s0, long long sk, int R) {
-  PFN_cuTensorMapEncodeTiled enc = encode_fn();
-  SidePlan pl;
-  if (!enc || !plan_side(&pl, side, kmajor, ptr, rows, K, inner, s1, s0, sk, R)) return false;
+bool encode(CUtensorMap* map, const c128* ptr, const SidePlan& pl) {
   cuuint32_t estr[4] = {1, 1, 1, 1};
-  const CUresult rc = enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 4, const_cast<c128*>(ptr), pl.dims, pl.strides, pl.box, estr,
-                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  const CUresult rc = encode_fn()(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 4, const_cast<c128*>(ptr), pl.dims, pl.strides, pl.box, estr,
+                                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   return rc == CUDA_SUCCESS;
 }
 
@@ -543,100 +332,38 @@ cudaError_t configure_tma() {
   return cudaFuncSetAttribute(zgemm_tma_kernel<C, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES);
 }
 
-// N <= 32 and enough rows to fill the machine with 256-row tiles: the tall geometry
-inline bool use_tall(const GemmDesc& d) { return d.N <= 32 && d.M >= 256 * 148; }
-
 }  // namespace
 
-cudaError_t zgemm_tma_configure_device() {
+cudaError_t zgemm_tma_configure_device(GemmCtx& ctx) {
+  ctx.tma_encode = encode_fn() != nullptr;
   cudaError_t e;
   if ((e = configure_tma<WideCfg>())) return e;
   return configure_tma<TallCfg>();
 }
 
-// Shape test only (no driver call): can both operands of `d` be described by tensor maps?  Used by the launch cost model.
-bool zgemm_tma_eligible(const GemmDesc& d) {
-  if (d.batch != 1 || d.M <= 0 || d.N <= 0 || d.K < BK || !encode_fn()) return false;
-  SidePlan pl;
-  TmaSide side;
-  bool km;
-  const int bm = use_tall(d) ? TallCfg::BM : WideCfg::BM, bn = use_tall(d) ? TallCfg::BN : WideCfg::BN;
-  return plan_side(&pl, &side, &km, d.A, d.M, d.K, d.a_m_inner, d.a_m1, d.a_m0, d.a_k, bm) &&
-         plan_side(&pl, &side, &km, d.B, d.N, d.K, d.b_n_inner, d.b_n1, d.b_n0, d.b_k, bn);
-}
-
-// Launch `d` (split-K fields already resolved by zgemm_auto) on the TMA kernel.  *used = false (and cudaSuccess) when the
-// shape is not expressible; nothing has been launched then.
-cudaError_t zgemm_tma_try(const GemmDesc& d, const GemmCtx& ctx, bool* used) {
-  *used = false;
-  if (d.batch != 1 || d.M <= 0 || d.N <= 0 || d.K < BK) return cudaSuccess;
-  if (d.splitk > 1 && (d.k_chunk % BK) != 0) return cudaSuccess;
+cudaError_t zgemm_tma_launch(const GemmDesc& d, const GemmPlan& pl, const GemmCtx& ctx) {
   CUtensorMap ma, mb;
+  if (!encode(&ma, d.A, pl.a_map) || !encode(&mb, d.B, pl.b_map)) return zgemm_dmma_launch(GEMM_BIG, d, ctx.stream);
   TmaParams p;
-  bool ak = false, bk = false;
-  const bool tall = use_tall(d);
-  const int BM = tall ? TallCfg::BM : WideCfg::BM, BN = tall ? TallCfg::BN : WideCfg::BN;
-  if (!make_side(&ma, &p.a, &ak, d.A, d.M, d.K, d.a_m_inner, d.a_m1, d.a_m0, d.a_k, BM)) return cudaSuccess;
-  if (!make_side(&mb, &p.b, &bk, d.B, d.N, d.K, d.b_n_inner, d.b_n1, d.b_n0, d.b_k, BN)) return cudaSuccess;
   p.M = d.M; p.N = d.N; p.K = d.K;
-  p.tiles_m = (d.M + BM - 1) / BM;
-  p.tiles_n = (d.N + BN - 1) / BN;
-  // group of M-tiles whose A rows (group_m * BM * K complex) take ~32 MB: they stay in L2 while the group walks the N-tiles,
-  // so B is read once per group.  ncu sweep on 8192 x 4096 x 1024 (algorithmic reads 201 MB): 693 / 617 / 778 / 1738 MB of
-  // DRAM reads for 16 / 32 / 48 / 64 MB groups -- the two L2 partitions duplicate lines that SMs of both dies read, so the
-  // usable capacity for an operand shared by all CTAs is about half of the 126 MB
-  {
-    const double a_tile_bytes = (double)BM * (double)d.K * 16.0;
-    int gm = (int)(32.0e6 / a_tile_bytes);
-    p.group_m = gm < 8 ? 8 : (gm > 64 ? 64 : gm);
-  }
-  p.splitk = d.splitk < 1 ? 1 : d.splitk;
-  p.k_chunk = d.k_chunk;
+  p.tiles_m = pl.tiles_m; p.tiles_n = pl.tiles_n; p.group_m = pl.group_m;
+  p.splitk = d.splitk; p.k_chunk = d.k_chunk;
+  p.a = pl.a; p.b = pl.b;
   p.a_conj = d.a_conj ? 1u : 0u;
   p.b_conj = d.b_conj ? 1u : 0u;
   p.C = d.C; p.c_m_inner = d.c_m_inner; p.c_m1 = d.c_m1; p.c_m0 = d.c_m0; p.c_n = d.c_n; p.c_split = d.c_split;
   p.alpha = d.alpha; p.beta = d.beta; p.c_stream = d.c_stream;
-  const long long total = (long long)p.tiles_m * p.tiles_n * p.splitk;
-  if (total > (1ll << 30)) return cudaSuccess;
-  int grid = (int)(total < ctx.num_sms ? total : ctx.num_sms);
-  // stream-K whenever whole tiles would leave a ragged last round -- or between half as many tiles as SMs and all of them:
-  // the ranges are then shorter than a tile and a tile's sums pass from one CTA to the next (this replaces split-K + its
-  // reduction kernel for these shapes).  The kernel handles chains of any length, but each link costs ~4 us (128 KB out,
-  // fence, flag, 128 KB in), so with fewer tiles than that the chain loses to split-K (measured: 8 tiles x 80 k-tiles ->
-  // 114 us against 47 us, profiles/r2_zgemm_shapes_auto_chain.jsonl) and is not used.  Short K (< 16 k-tiles: H_eff stage
-  // 2) loses more to the fix-up than it gains; force_cfg 5 = TMA kernel with whole tiles only (A/B tests)
-  const int KT = (d.K + BK - 1) / BK;
-  p.streamk = 0;
-  p.sk_tiles = (int)total;
-  if (p.splitk == 1 && ctx.force_cfg != 5 && ctx.sk_ws && ctx.sk_flags && KT >= 16 && ctx.num_sms <= ctx.sk_slots) {
-    if (total >= ctx.num_sms) {
-      // only when the ragged last wave costs more than 3 %: with many waves stream-K gains nothing measurable and its
-      // k-shifted first waves cost L2 reuse (8192 x 4096 x 1024, 27.7 waves: 617 MB of DRAM reads with, 522 MB without)
-      const long long waves = (total + ctx.num_sms - 1) / ctx.num_sms;
-      p.streamk = ((waves * ctx.num_sms - total) * 100 > 3 * waves * ctx.num_sms || ctx.force_cfg == 4) ? 1 : 0;
-      if (total % ctx.num_sms == 0) p.streamk = 0;
-      p.sk_tiles = (int)(total % ctx.num_sms) + (total >= 2 * ctx.num_sms ? ctx.num_sms : 0);   // one to two waves' worth
-      if (total < 2 * ctx.num_sms) p.sk_tiles = (int)total;
-    } else {
-      p.sk_tiles = (int)total;
-      if (2 * total >= ctx.num_sms && KT >= 32) { p.streamk = 1; grid = ctx.num_sms; }   // <= 2 links, >= 16 k-tiles each
-      else if (ctx.force_cfg == 4) {                      // forced "tma": long chains too (ranges of >= 4 k-tiles), for the tests
-        long long g = total * KT / 4;
-        if (g > ctx.num_sms) g = ctx.num_sms;
-        if (g > total) { p.streamk = 1; grid = (int)g; }
-      }
-    }
-  }
+  p.streamk = pl.streamk; p.sk_tiles = pl.sk_tiles;
   p.sk_flags = ctx.sk_flags;
   p.sk_ws = ctx.sk_ws;
   p.epoch = p.streamk ? ++ctx.sk_epoch : 0;
   cudaError_t e;
   {
     ProfScope scope(ctx.stream, d.tag, 8.0 * (double)d.M * (double)d.N * (double)d.K, true);
-    e = tall ? launch_tma<TallCfg>(ak, bk, ma, mb, p, grid, ctx.stream) : launch_tma<WideCfg>(ak, bk, ma, mb, p, grid, ctx.stream);
+    e = pl.kernel == GEMM_TMA_TALL ? launch_tma<TallCfg>(pl.a_kmajor, pl.b_kmajor, ma, mb, p, pl.grid, ctx.stream)
+                                   : launch_tma<WideCfg>(pl.a_kmajor, pl.b_kmajor, ma, mb, p, pl.grid, ctx.stream);
   }
   count_launch();
-  *used = true;
   return e;
 }
 
