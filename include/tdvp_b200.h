@@ -129,7 +129,8 @@ int tdvp_lanczos_eigvec(tdvp_handle_t h, const tdvp_heff_term* hterms, int nterm
 /* ---- gauge shift ------------------------------------------------------------------------------- */
 /* Householder QR with LAPACK zgeqrf/zungqr conventions -- replaces SiteCoef.gauge_trf
  * (pytdscf/_site_cls.py:138-292).  gauge A: psi(Dl,d,Dr) -> site(Dl,d,k), sigma(k,Dr);
- * gauge B: psi -> sigma(Dl,k), site(k,d,Dr); k = min(rows, cols) of the matricisation. */
+ * gauge B: psi -> sigma(Dl,k), site(k,d,Dr); k = min(rows, cols) of the matricisation.  The row count has no limit
+ * beyond the workspace: panels taller than num_sms x 256 rows keep their slabs in global memory. */
 int tdvp_qr_shift(tdvp_handle_t h, int gauge, int Dl, int d, int Dr, const tdvp_c128* psi,
                   tdvp_c128* site, tdvp_c128* sigma);
 /* gauge A: out(k,d,Dr) = sigma(k,Dl) . site(Dl,d,Dr);  gauge B: out(Dl,d,k) = site(Dl,d,Dr) . sigma(Dr,k)
@@ -148,7 +149,8 @@ int tdvp_svd_truncate(tdvp_handle_t h, int m, int n, const tdvp_c128* sigma, dou
                       tdvp_c128* U, tdvp_c128* S, tdvp_c128* Vh, int* rank);
 /* Thin SVD A(m,n) = U(m,n) diag(s) Vh(n,n), m >= n, s descending and written to HOST memory -- replaces
  * np.linalg.svd / scipy.linalg.svd in CC2ALambdaB (pytdscf/_mps_cls.py:3601-3630) and in the regularised gauge_trf
- * (pytdscf/_site_cls.py:207-252). */
+ * (pytdscf/_site_cls.py:207-252).  Any m >= n: zero singular values get their left vectors from a Householder QR,
+ * which has no row limit (see tdvp_qr_shift). */
 int tdvp_svd(tdvp_handle_t h, int m, int n, const tdvp_c128* A, tdvp_c128* U, double* s_host, tdvp_c128* Vh);
 /* out(n,m) = pinv(X(m,n), rcond) -- replaces np.linalg.pinv in multiply_sigvec_pinv (pytdscf/_site_cls.py:734). */
 int tdvp_pinv(tdvp_handle_t h, int m, int n, const tdvp_c128* X, double rcond, tdvp_c128* out);

@@ -11,7 +11,8 @@
 // zlarft and the zlarfb block applications; only summation order differs from LAPACK.
 //
 // Panel factorisation (k_qr_panel): a cooperative kernel, one CTA per slab of <= SLAB_ROWS rows, the slab of
-// the 32-column panel lives in shared memory for the whole panel.  Per column ONE grid-wide reduction gives
+// the 32-column panel lives in shared memory for the whole panel.  A panel taller than num_sms x SLAB_ROWS rows gets
+// one CTA per SM with ceil(rows / num_sms) rows each, and the slabs then live in a global-memory buffer instead.  Per column ONE grid-wide reduction gives
 // both |x|^2 and every v^H a_j: with g_j = sum_{i>c} conj(a_ic) a_ij,  w_j = a_cj + conj(s) g_j where
 // s = 1/(alpha - beta).  Partials are combined in fixed CTA order (deterministic).  Trailing updates and the
 // formation of Q are DMMA ZGEMMs on explicit unit-lower-trapezoidal V panels.
@@ -38,6 +39,7 @@ struct PanelArgs {
   double* gpart;   // 2 buffers x G x (2*NB complex): [buf][cta][0..NB) partial g, [NB..2NB) diagonal row broadcast
   double* zpart;   // G x NB x NB complex partial Gram for T
   int rows_per_cta;
+  c128* gslab;     // k_qr_panel only: nullptr = slabs in shared memory, else [G][rows_per_cta][NB] in global memory
   int dbg;         // timing experiments only (TDVP_QR_DEBUG): bit 0 skips the column loop, bit 1 the T factor
 };
 
@@ -50,7 +52,8 @@ __device__ __forceinline__ double dlapy3(double x, double y, double z) {
 
 __global__ void __launch_bounds__(PT, 1) k_qr_panel(PanelArgs p) {
   extern __shared__ __align__(16) unsigned char smraw[];
-  c128* S = reinterpret_cast<c128*>(smraw);                 // [rows_per_cta][NB]
+  // [rows_per_cta][NB]; only this CTA touches its slab, so __syncthreads orders the global-memory variant too
+  c128* S = p.gslab ? p.gslab + (size_t)blockIdx.x * p.rows_per_cta * NB : reinterpret_cast<c128*>(smraw);
   __shared__ c128 red[PTY][NB];
   __shared__ c128 gtot[NB];     // reduced g_j
   __shared__ c128 rowc[NB];     // row c of the panel (broadcast)
@@ -574,7 +577,7 @@ constexpr int QR_MAX_SMS = 256;  // workspace bound for the per-CTA partials (B2
 
 size_t qr_ws_elems(int m, int n) {
   const size_t np = (n + NB - 1) / NB;
-  return 3 * (size_t)m * n + np * NB * NB + 2 * (size_t)NB * n + 4096 + (size_t)QR_MAX_SMS * NB * NB + QR_MAX_SMS * 4 * NB;
+  return 3 * (size_t)m * n + (size_t)(m + QR_MAX_SMS) * NB + np * NB * NB + 2 * (size_t)NB * n + 4096 + (size_t)QR_MAX_SMS * NB * NB + QR_MAX_SMS * 4 * NB;
 }
 
 // Per-device kernel attributes and co-scheduling limits of the panel kernels (tdvp_create, once per handle).
@@ -615,7 +618,12 @@ int qr_factor(Handle* h, c128* A, int m, int n, int lda, c128* Q, int ldq) {
   double* tau = (double*)ws_alloc(h, sizeof(double) * 2 * (size_t)n);
   double* gpart = (double*)ws_alloc(h, sizeof(double) * 2 * (size_t)max_coop * 4 * NB);
   double* zpart = (double*)ws_alloc(h, sizeof(double) * 2 * (size_t)max_coop * NB * NB);
-  if (!Vall || !Tall || !W || !W2 || !tau || !gpart || !zpart) { set_error(h, "qr_factor: workspace"); return TDVP_ERR_ARG; }
+  // slabs of the panels taller than max_coop x SLAB_ROWS rows (the first panel is the tallest); G x rpc <= m + G rows
+  c128* gslab = (m > max_coop * SLAB_ROWS) ? (c128*)ws_alloc(h, sizeof(c128) * (size_t)(m + max_coop) * NB) : nullptr;
+  if (!Vall || !Tall || !W || !W2 || !tau || !gpart || !zpart || (m > max_coop * SLAB_ROWS && !gslab)) {
+    set_error(h, "qr_factor: workspace");
+    return TDVP_ERR_ARG;
+  }
   TDVP_CUDA(h, cudaMemsetAsync(Vall, 0, sizeof(c128) * (size_t)m * lda, h->stream));
   const c128 one = {1.0, 0.0}, zero = {0.0, 0.0}, mone = {-1.0, 0.0};
 
@@ -631,7 +639,7 @@ int qr_factor(Handle* h, c128* A, int m, int n, int lda, c128* Q, int ldq) {
       while (G < max_cluster && (mp + G - 1) / G > rows_target) G *= 2;
       while ((mp + G - 1) / G > CL_ROWS) G *= 2;
       const int rpc = (mp + G - 1) / G;
-      PanelArgs pa{A, lda, m, n, j0, jb, tau, Vall, Tall, gpart, zpart, rpc, qr_dbg};
+      PanelArgs pa{A, lda, m, n, j0, jb, tau, Vall, Tall, gpart, zpart, rpc, nullptr, qr_dbg};
       cudaLaunchConfig_t cfg = {};
       cfg.gridDim = dim3(G);
       cfg.blockDim = dim3(32, CTY);
@@ -647,12 +655,13 @@ int qr_factor(Handle* h, c128* A, int m, int n, int lda, c128* Q, int ldq) {
     } else {
       int rpc = SLAB_ROWS;
       int G = (mp + rpc - 1) / rpc;
-      if (G > max_coop) { set_error(h, "qr_factor: matrix too tall for the cooperative panel kernel"); return TDVP_ERR_UNSUPPORTED; }
+      const bool global_slabs = G > max_coop;   // more slabs than SMs: one CTA per SM, slabs in global memory
+      if (global_slabs) G = max_coop;
       if (G < 1) G = 1;
       rpc = (mp + G - 1) / G;  // spread rows evenly
-      PanelArgs pa{A, lda, m, n, j0, jb, tau, Vall, Tall, gpart, zpart, rpc, qr_dbg};
+      PanelArgs pa{A, lda, m, n, j0, jb, tau, Vall, Tall, gpart, zpart, rpc, global_slabs ? gslab : nullptr, qr_dbg};
       void* args[] = {&pa};
-      const size_t smem = sizeof(c128) * (size_t)(rpc > 2 * NB ? rpc : 2 * NB) * NB;
+      const size_t smem = global_slabs ? 0 : sizeof(c128) * (size_t)(rpc > 2 * NB ? rpc : 2 * NB) * NB;
       { ProfScope _ps(h->stream, "qr.k_qr_panel"); e = cudaLaunchCooperativeKernel((void*)k_qr_panel, dim3(G), dim3(32, PTY), args, smem, h->stream); }
       count_launch();
       if (e != cudaSuccess) return cuda_fail(h, e, "cudaLaunchCooperativeKernel(k_qr_panel)", __FILE__, __LINE__);

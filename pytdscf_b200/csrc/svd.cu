@@ -11,7 +11,9 @@
 // the round-robin tournament are independent and are spread over the CTAs of a cooperative grid (one grid sync per
 // round).  One-sided Jacobi orthogonalises tiny columns to THEIR OWN scale (high relative accuracy), so U stays
 // unitary down to the smallest non-zero singular value; exactly-zero columns are completed by a Householder QR of
-// the padded matrix (the same LAPACK-style null-space completion the gauge shift uses).
+// the padded matrix (the same LAPACK-style null-space completion the gauge shift uses).  That QR takes any row count, so
+// tall rank-deficient inputs such as the (D_l D_r) x d matricisation of regularize_site with an empty physical level
+// are completed too (above num_sms x 256 rows its panel slabs live in global memory).
 #include <cooperative_groups.h>
 
 #include <algorithm>

@@ -146,30 +146,52 @@ def test_env_update_summed_block_and_accumulate(eng, K):
     assert relerr(out.cpu().numpy(), ref) < 1e-13
 
 
+ENV_SHAPES = [(37, 5, 29, 3, 4), (64, 10, 48, 6, 6), (130, 4, 70, 2, 5)]
+
+
 @pytest.mark.parametrize("gauge", ["A", "B"])
-@pytest.mark.parametrize("Dl,d,Dr,wi,wo", [(37, 5, 29, 3, 4), (64, 10, 48, 6, 6), (130, 4, 70, 2, 5)])
-def test_env_update_random_shapes(eng, gauge, Dl, d, Dr, wi, wo):
+@pytest.mark.parametrize("Dl,d,Dr,wi,wo,bra_ket,diag",
+                         [pytest.param(*s, "same", False, id="-".join(map(str, s))) for s in ENV_SHAPES] +
+                         [pytest.param(*s, "independent", diag, id="-".join(map(str, s)) + ("-bra-diag" if diag else "-bra"))
+                          for s in ENV_SHAPES for diag in (False, True)])
+def test_env_update_random_shapes(eng, gauge, Dl, d, Dr, wi, wo, bra_ket, diag):
+    """bra == ket, and independent bra and ket (Simulator.operate, adaptive mode): a swap of the two would show."""
     rng = np.random.default_rng(Dl + 3 * d + 5 * Dr + wi + wo)
     A = crand(rng, Dl, d, Dr)
+    shape_W = ((wi, d, wo) if gauge == "A" else (wo, d, wi)) if diag else ((wi, d, d, wo) if gauge == "A" else (wo, d, d, wi))
     if gauge == "A":
-        E, W = crand(rng, Dl, wi, Dl), crand(rng, wi, d, d, wo)
+        E, W = crand(rng, Dl, wi, Dl), crand(rng, *shape_W)
     else:
-        E, W = crand(rng, Dr, wi, Dr), crand(rng, wo, d, d, wi)
-    ref = orc.env_update_term(gauge, A, A, E, core_of(W))
-    out = eng.env_update(gauge, eng.to_device(A), eng.to_device(A), eng.to_device(E), eng.upload_core(W))
+        E, W = crand(rng, Dr, wi, Dr), crand(rng, *shape_W)
+    bra = A if bra_ket == "same" else crand(rng, Dl, d, Dr)
+    ref = orc.env_update_term(gauge, bra, A, E, core_of(W))
+    out = eng.env_update(gauge, eng.to_device(bra), eng.to_device(A), eng.to_device(E), eng.upload_core(W))
     assert relerr(out.cpu().numpy(), ref) < 1e-12
 
 
 # ---------------------------------------------------------------------------------------------
-def _check_qr(eng, psi, atol=1e-12):
-    A, s = orc.shift_qr(psi)
-    Ad, sd = eng.qr_shift("A", eng.to_device(psi))
-    np.testing.assert_allclose(Ad.cpu().numpy(), A, atol=atol)
-    np.testing.assert_allclose(sd.cpu().numpy(), s, atol=atol * max(1.0, np.abs(s).max()))
-    s, B = orc.shift_lq(psi)
-    Bd, sd = eng.qr_shift("B", eng.to_device(psi))
-    np.testing.assert_allclose(Bd.cpu().numpy(), B, atol=atol)
-    np.testing.assert_allclose(sd.cpu().numpy(), s, atol=atol * max(1.0, np.abs(s).max()))
+def _check_qr(eng, psi, atol=1e-12, gauges="AB"):
+    """Gauge A on psi and gauge B on psi.  Besides the elementwise match with LAPACK: Q^H Q = I and QR = psi to 1e-13
+    (~ 450 EPS: Householder orthogonality and backward error are a small multiple of sqrt(rows) EPS up to 37888 rows)."""
+    Dl, d, Dr = psi.shape
+    if "A" in gauges:
+        A, s = orc.shift_qr(psi)
+        Ad, sd = eng.qr_shift("A", eng.to_device(psi))
+        Ad, sd = Ad.cpu().numpy(), sd.cpu().numpy()
+        np.testing.assert_allclose(Ad, A, atol=atol)
+        np.testing.assert_allclose(sd, s, atol=atol * max(1.0, np.abs(s).max()))
+        Q = Ad.reshape(Dl * d, Dr)
+        assert np.abs(Q.conj().T @ Q - np.eye(Dr)).max() <= 1e-13
+        assert np.linalg.norm(Q @ sd - psi.reshape(Dl * d, Dr)) <= 1e-13 * np.linalg.norm(psi)
+    if "B" in gauges:
+        s, B = orc.shift_lq(psi)
+        Bd, sd = eng.qr_shift("B", eng.to_device(psi))
+        Bd, sd = Bd.cpu().numpy(), sd.cpu().numpy()
+        np.testing.assert_allclose(Bd, B, atol=atol)
+        np.testing.assert_allclose(sd, s, atol=atol * max(1.0, np.abs(s).max()))
+        Q = Bd.reshape(Dl, d * Dr)
+        assert np.abs(Q @ Q.conj().T - np.eye(Dl)).max() <= 1e-13
+        assert np.linalg.norm(sd @ Q - psi.reshape(Dl, d * Dr)) <= 1e-13 * np.linalg.norm(psi)
 
 
 def test_qr_shift_golden(eng, K):
@@ -191,10 +213,27 @@ def test_qr_shift_zero_padded_matches_lapack_completion(eng, K):
     np.testing.assert_allclose(sd.cpu().numpy(), K["g_padBsig"], atol=1e-14)
 
 
-@pytest.mark.parametrize("Dl,d,Dr", [(1, 8, 4), (4, 8, 4), (16, 5, 16), (40, 6, 40), (64, 10, 64), (100, 7, 90), (128, 16, 128)])
+# Tall matricisations (rows, 1, cols) at the QR panel kernels' switch points: k_qr_panel_cluster with 1 CTA (64 rows),
+# 2 CTAs (65, 128), 16 CTAs (1024), the last cluster size (4096 = 16 x 256 rows); k_qr_panel above (4097, 8192, 20000),
+# its widest grid with shared-memory slabs ("sms": num_sms x 256 rows) and the first size with global-memory slabs.
+QR_TALL_ROWS = [64, 65, 128, 1024, 4096, 4097, 8192, 20000, "sms", "sms+1"]
+QR_TALL_COLS = [1, 31, 32, 33, 100]
+
+
+@pytest.mark.parametrize("Dl,d,Dr", [(1, 8, 4), (4, 8, 4), (16, 5, 16), (40, 6, 40), (64, 10, 64), (100, 7, 90), (128, 16, 128)] +
+                         [(rows, 1, cols) for rows in QR_TALL_ROWS for cols in QR_TALL_COLS if rows == "sms" or rows == "sms+1" or cols <= rows])
 def test_qr_shift_random(eng, Dl, d, Dr):
+    if isinstance(Dl, str):
+        import torch
+
+        Dl = torch.cuda.get_device_properties(0).multi_processor_count * 256 + (Dl == "sms+1")
     rng = np.random.default_rng(Dl * 100 + d * 10 + Dr)
-    _check_qr(eng, crand(rng, Dl, d, Dr))
+    psi = crand(rng, Dl, d, Dr)
+    if Dl <= Dr * d:
+        _check_qr(eng, psi)
+    else:   # gauge B factors the same (rows x cols) matrix when given the transposed tensor
+        _check_qr(eng, psi, gauges="A")
+        _check_qr(eng, np.ascontiguousarray(psi.transpose(2, 1, 0)), gauges="B")
 
 
 def test_qr_shift_partial_rank(eng):
