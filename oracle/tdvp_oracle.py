@@ -242,10 +242,12 @@ def _rescale(y, b0, conserve_norm):
     return y * b0
 
 
-def sil_reference(scale, matvec, psi, thresh, *, last_niter=0, conserve_norm=True, maxsize=None):
+def sil_reference(scale, matvec, psi, thresh, *, last_niter=0, conserve_norm=True, maxsize=None, small_expm=None):
     """exp(scale*H) psi by the reference's three-term recurrence (alpha_l = <v0|H v_l>).
 
-    ``matvec`` maps an array of ``psi.shape`` to one of the same shape.  Returns (psi_new, niter)."""
+    ``matvec`` maps an array of ``psi.shape`` to one of the same shape.  Returns (psi_new, niter).
+    ``small_expm``: optional callable A -> expm(A)[:, 0] for the k x k matrix A = scale * T (k >= 2) that replaces the
+    reference's eigh_tridiagonal / eig step, e.g. a high-precision exponential; None keeps the reference's arithmetic."""
     shape = psi.shape
     maxsize = psi.size if maxsize is None else int(maxsize)   # adaptive runs: size of the tensor before it was extended
     ndim, n_warm = krylov_warmup(maxsize, last_niter)
@@ -286,6 +288,13 @@ def sil_reference(scale, matvec, psi, thresh, *, last_niter=0, conserve_norm=Tru
             continue
         if l == 0:
             y = v0 * cmath.exp(scale * alpha[0])
+        elif small_expm is not None:
+            T = (
+                np.diag(np.real(alpha) if alpha_is_real else np.asarray(alpha), 0).astype(np.complex128)
+                + np.diag(beta[:-1], -1)
+                + np.diag(beta[:-1], 1)
+            )
+            y = np.dot(small_expm(scale * T), np.asarray(V[:-1]))
         else:
             if alpha_is_real:
                 lam, phi = scipy.linalg.eigh_tridiagonal(np.real(alpha), beta[:-1])
@@ -309,8 +318,9 @@ def sil_reference(scale, matvec, psi, thresh, *, last_niter=0, conserve_norm=Tru
     raise ValueError("Short Iterative Lanczos is not converged")
 
 
-def sia_reference(scale, matvec, psi, thresh, *, last_niter=0, conserve_norm=True, maxsize=None):
-    """Arnoldi variant: one-pass classical Gram-Schmidt, dense eig of the Hessenberg block."""
+def sia_reference(scale, matvec, psi, thresh, *, last_niter=0, conserve_norm=True, maxsize=None, small_expm=None):
+    """Arnoldi variant: one-pass classical Gram-Schmidt, dense eig of the Hessenberg block (``small_expm`` as in
+    ``sil_reference``, applied to scale times the Hessenberg block)."""
     shape = psi.shape
     maxsize = psi.size if maxsize is None else int(maxsize)
     ndim, n_warm = krylov_warmup(maxsize, last_niter)
@@ -347,6 +357,9 @@ def sia_reference(scale, matvec, psi, thresh, *, last_niter=0, conserve_norm=Tru
             continue
         if l == 0:
             y = v0 * cmath.exp(scale * hess[0, 0])
+        elif small_expm is not None:
+            c = small_expm(scale * hess[: l + 1, : l + 1])
+            y = np.tensordot(c, V[: c.shape[0], :], axes=(0, 0))
         else:
             sub = hess[: l + 1, : l + 1]
             lam, phi = np.linalg.eig(sub)
