@@ -174,4 +174,8 @@ int tdvp_zgemm(tdvp_handle_t h, int transA, int transB, int M, int N, int K, dou
 #ifdef __cplusplus
 }
 #endif
+
+/* two-site TDVP entry points (same conventions, same ABI version) */
+#include "tdvp_b200_two_site.h"
+
 #endif /* TDVP_B200_H */

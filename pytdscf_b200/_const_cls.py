@@ -24,6 +24,9 @@ class RunConfig:
     dD: int = 5          # adaptive_dD
     p_proj: float = 1.0e-04  # adaptive_p_proj
     p_svd: float = 1.0e-07  # adaptive_p_svd: truncation weight of the site-parallel boundary bond (reference const.p_svd)
+    two_site: bool = False  # two-site TDVP: bonds follow the state (truncated SVD split of every pair)
+    two_site_p_svd: float = 1.0e-07  # truncation weight of the two-site split (the rule of adaptive_p_svd)
+    bond_dim: int = 0  # two-site TDVP: bond-dimension cap (the model's bond_dim; 0 = matricisation ranks only)
 
     def __post_init__(self):
         self.space = self.space.lower()
@@ -36,3 +39,5 @@ class RunConfig:
             self.conserve_norm = False
         if self.adaptive and self.relax:
             raise NotImplementedError("adaptive bond dimensions are implemented for real-time propagation only")
+        if self.two_site and (self.relax or self.adaptive):
+            raise NotImplementedError("two-site TDVP is implemented for real-time propagation without adaptive=True")

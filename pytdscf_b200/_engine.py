@@ -12,7 +12,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import GAUGE_A, GAUGE_B, KIND_DIAG, KIND_FULL, HeffTerm, KeffTerm, check
+from ._lib import GAUGE_A, GAUGE_B, KIND_DIAG, KIND_FULL, Heff2Term, HeffTerm, KeffTerm, check
 
 CDTYPE = torch.complex128
 
@@ -149,7 +149,42 @@ class Engine:
             t.coef_re, t.coef_im = c.real, c.imag
         return arr
 
+    def heff2_terms(self, terms):
+        """Two-site terms: iterable of (L | None, DeviceCore | None, DeviceCore | None, R | None, coef) -- a None core is the
+        identity on that site (a key that acts on the other site only)."""
+        arr = (Heff2Term * len(terms))()
+        for i, (L, c1, c2, R, coef) in enumerate(terms):
+            t = arr[i]
+            c1 = None if c1 is None or c1.data is None else c1
+            c2 = None if c2 is None or c2.data is None else c2
+            t.L = None if L is None else L.data_ptr()
+            t.R = None if R is None else R.data_ptr()
+            t.wl = 1 if L is None else int(L.shape[1])
+            t.wr = 1 if R is None else int(R.shape[1])
+            t.wm = c1.wr if c1 is not None else (c2.wl if c2 is not None else 1)
+            if c1 is not None and (c1.wl != t.wl or (c2 is not None and c2.wl != c1.wr)) or c2 is not None and c2.wr != t.wr:
+                raise ValueError("two-site term: block / core bond dimensions do not match")
+            for c, W, Wp, kind in ((c1, "W1", "W1p", "w1_kind"), (c2, "W2", "W2p", "w2_kind")):
+                setattr(t, W, None if c is None else c.data.data_ptr())
+                setattr(t, Wp, None if c is None or c.perm is None else c.perm.data_ptr())
+                setattr(t, kind, _lib.KIND_IDENTITY if c is None else c.kind)
+            l_id = c1.l_id if c1 is not None and L is not None else -1
+            r_id = c2.r_id if c2 is not None and R is not None else -1
+            t.id_channels = (l_id + 1) | ((r_id + 1) << 16)
+            c = complex(coef)
+            t.coef_re, t.coef_im = c.real, c.imag
+        return arr
+
     # -- contractions ----------------------------------------------------------------
+    def heff2_apply(self, terms, theta: torch.Tensor) -> torch.Tensor:
+        """out(Dl,d1,d2,Dr) = H2 theta for the two-site terms of ``heff2_terms``."""
+        _chk_tensor(theta, "theta")
+        Dl, d1, d2, Dr = theta.shape
+        out = torch.empty_like(theta)
+        arr = self.heff2_terms(terms)
+        check(self.h, self.lib.tdvp_heff2_apply(self.h, arr, len(terms), Dl, d1, d2, Dr, _ptr(theta), _ptr(out)))
+        return out
+
     def heff_apply(self, terms, psi: torch.Tensor) -> torch.Tensor:
         _chk_tensor(psi, "psi")
         Dl, d, Dr = psi.shape
@@ -215,6 +250,20 @@ class Engine:
                                            int(bool(conserve_norm)), None, arr, len(kterms), Dl, 1, Dr, _ptr(psi),
                                            C.byref(niter))
         check(self.h, rc)
+        return int(niter.value)
+
+    def krylov_expm2(self, kind: str, scale: complex, thresh: float, n_warmup: int, conserve_norm: bool,
+                     theta: torch.Tensor, terms) -> int:
+        """theta(Dl,d1,d2,Dr) <- exp(scale*H2) theta in place; returns the number of Krylov vectors used."""
+        _chk_tensor(theta, "theta")
+        k = _lib.KRYLOV_ARNOLDI if kind == "arnoldi" else _lib.KRYLOV_LANCZOS_REF
+        niter = C.c_int(0)
+        scale = complex(scale)
+        Dl, d1, d2, Dr = theta.shape
+        arr = self.heff2_terms(terms)
+        check(self.h, self.lib.tdvp_krylov_expm2(self.h, k, scale.real, scale.imag, float(thresh), int(n_warmup),
+                                                 int(bool(conserve_norm)), arr, len(terms), Dl, d1, d2, Dr, _ptr(theta),
+                                                 C.byref(niter)))
         return int(niter.value)
 
     def lanczos_eigvec(self, psi: torch.Tensor, hterms, root: int = 0, thresh: float = 1e-9) -> int:
@@ -286,6 +335,21 @@ class Engine:
         if keepdim:
             return U, S, Vh, r
         return U[:, :r].contiguous(), S.reshape(-1)[: r * r].reshape(r, r), Vh[:r, :].contiguous(), r
+
+    def split2(self, direction: str, theta: torch.Tensor, p: float, Dcap: int, conserve_norm: bool):
+        """Truncated split of theta(Dl,d1,d2,Dr): direction "right" -> (A(Dl,d1,r), centre(r,d2,Dr)), "left" ->
+        (centre(Dl,d1,r), B(r,d2,Dr)); returns (left, right, s (host float64, all singular values), r)."""
+        _chk_tensor(theta, "theta")
+        Dl, d1, d2, Dr = theta.shape
+        k = max(1, min(int(Dcap), Dl * d1, d2 * Dr))
+        left, right = self.empty(Dl * d1 * k), self.empty(k * d2 * Dr)
+        s = (C.c_double * min(Dl * d1, d2 * Dr))()
+        rank = C.c_int(0)
+        g = GAUGE_A if direction == "right" else GAUGE_B
+        check(self.h, self.lib.tdvp_split2(self.h, g, Dl, d1, d2, Dr, _ptr(theta), float(p), k, int(bool(conserve_norm)),
+                                           _ptr(left), _ptr(right), s, C.byref(rank)))
+        r = int(rank.value)
+        return (left[: Dl * d1 * r].view(Dl, d1, r), right[: r * d2 * Dr].view(r, d2, Dr), np.array(s[:], dtype=np.float64), r)
 
     def svd(self, M: torch.Tensor):
         """Thin SVD of a 2-D tensor: (U, s (host float64 array), Vh); wide matrices go through the conjugate transpose."""

@@ -46,6 +46,16 @@ class KeffTerm(C.Structure):
     ]
 
 
+class Heff2Term(C.Structure):
+    _fields_ = [
+        ("L", C.c_void_p), ("W1", C.c_void_p), ("W1p", C.c_void_p), ("W2", C.c_void_p), ("W2p", C.c_void_p),
+        ("R", C.c_void_p), ("wl", C.c_int32), ("wm", C.c_int32), ("wr", C.c_int32), ("w1_kind", C.c_int32),
+        ("w2_kind", C.c_int32), ("id_channels", C.c_int32), ("coef_re", C.c_double), ("coef_im", C.c_double),
+    ]
+
+
+ERR_NO_MEMORY = -6
+
 # name -> (restype, argtypes); must list every symbol include/tdvp_b200.h declares
 SIGNATURES = {
     "tdvp_abi_version": (C.c_int, []),
@@ -81,6 +91,17 @@ SIGNATURES = {
                              C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_double, C.c_double, C.c_void_p, C.c_int]),
 }
 
+# the two-site entry points of include/tdvp_b200_two_site.h
+SIGNATURES_TWO_SITE = {
+    "tdvp_heff2_apply": (C.c_int, [C.c_void_p, C.POINTER(Heff2Term), C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                   C.c_void_p, C.c_void_p]),
+    "tdvp_krylov_expm2": (C.c_int, [C.c_void_p, C.c_int, C.c_double, C.c_double, C.c_double, C.c_int, C.c_int,
+                                    C.POINTER(Heff2Term), C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                    C.POINTER(C.c_int)]),
+    "tdvp_split2": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_double, C.c_int,
+                              C.c_int, C.c_void_p, C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_int)]),
+}
+
 _lib = None
 
 
@@ -95,7 +116,7 @@ def load_library():
             "(or __graft_entry__.build()).  There is no CPU fallback for backend='cuda'."
         )
     lib = C.CDLL(LIB_PATH)
-    for name, (res, args) in SIGNATURES.items():
+    for name, (res, args) in {**SIGNATURES, **SIGNATURES_TWO_SITE}.items():
         fn = getattr(lib, name)
         fn.restype = res
         fn.argtypes = args

@@ -599,6 +599,13 @@ class MPSCoefCuda:
         """One time step: forward and backward half sweeps (the last site gets two consecutive half steps); one-site
         gates and Kraus maps, if any, act between the two (reference ``_mps_cls.py:452-503``)."""
         n = self.nsite
+        if getattr(cfg, "two_site", False):
+            if one_gate is not None or kraus_op is not None:
+                raise NotImplementedError("two-site TDVP applies no gates or Kraus maps between its half sweeps")
+            from ._twosite import propagate_two_site
+
+            propagate_two_site(self, stepsize, H, cfg)
+            return
         self.propagate_along_sweep(H, stepsize, cfg, begin_site=0, end_site=n - 1)
         if one_gate is not None:
             self.apply_one_gate(one_gate, reorth_center=n - 1)

@@ -8,6 +8,9 @@ namespace tdvp {
 int krylov_expm_exec(Handle* h, int kind, double scale_re, double scale_im, double thresh, int n_warmup,
                      int conserve_norm, const tdvp_heff_term* hterms, const tdvp_keff_term* kterms, int nterms,
                      int Dl, int d, int Dr, c128* psi, int* niter);
+int krylov_expm2_exec(Handle* h, int kind, double scale_re, double scale_im, double thresh, int n_warmup,
+                      int conserve_norm, const tdvp_heff2_term* terms, int nterms, int Dl, int d1, int d2, int Dr, c128* theta,
+                      int* niter);
 int lanczos_eigvec_exec(Handle* h, const tdvp_heff_term* hterms, int nterms, int Dl, int d, int Dr, c128* psi, int root,
                         double thresh, int* niter);
 int inner_exec(Handle* h, long long n, const c128* bra, const c128* ket, int conj, c128* host_out);
@@ -57,6 +60,24 @@ int ws_grow_preserve(Handle* h, size_t bytes) {
   h->ws = (unsigned char*)p;
   h->ws_bytes = bytes;
   return 0;
+}
+
+int ws_reserve_checked(Handle* h, size_t bytes, const char* what) {
+  if (bytes <= h->ws_bytes) return ws_reserve(h, bytes);
+  auto fail = [&]() {
+    char buf[256];
+    snprintf(buf, sizeof(buf), "%s: the device workspace cannot grow to %.3f GB (%zu bytes)", what, bytes / 1.0e9, bytes);
+    set_error(h, buf);
+    return (int)TDVP_ERR_NO_MEMORY;
+  };
+  size_t free_b = 0, total_b = 0;
+  if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess && bytes > total_b) return fail();   // more than the device has: do not try
+  const int rc = ws_reserve(h, bytes);
+  if (rc == (int)cudaErrorMemoryAllocation) {
+    cudaGetLastError();   // an allocation failure is not sticky: clear it so later calls do not report it
+    return fail();
+  }
+  return rc;
 }
 
 void* ws_alloc(Handle* h, size_t bytes) {
@@ -194,6 +215,24 @@ int tdvp_heff_apply(tdvp_handle_t h, const tdvp_heff_term* terms, int nterms, in
   if (psi == out) { set_error(h, "heff_apply: out must not alias psi"); return TDVP_ERR_ARG; }
   TDVP_TRY(ws_reserve(h, sizeof(c128) * heff_ws_elems(terms, nterms, Dl, d, Dr)));
   return heff_apply_exec(h, terms, nterms, Dl, d, Dr, (const c128*)psi, (c128*)out);
+}
+
+int tdvp_heff2_apply(tdvp_handle_t h, const tdvp_heff2_term* terms, int nterms, int Dl, int d1, int d2, int Dr,
+                     const tdvp_c128* theta, tdvp_c128* out) {
+  H_CHECK(h);
+  if (!terms || !theta || !out || nterms <= 0 || Dl <= 0 || d1 <= 0 || d2 <= 0 || Dr <= 0) { set_error(h, "heff2_apply: bad argument"); return TDVP_ERR_ARG; }
+  if (theta == out) { set_error(h, "heff2_apply: out must not alias theta"); return TDVP_ERR_ARG; }
+  TDVP_TRY(ws_reserve_checked(h, sizeof(c128) * heff2_ws_elems(terms, nterms, Dl, d1, d2, Dr), "heff2_apply"));
+  return heff2_apply_exec(h, terms, nterms, Dl, d1, d2, Dr, (const c128*)theta, (c128*)out);
+}
+
+int tdvp_krylov_expm2(tdvp_handle_t h, int kind, double scale_re, double scale_im, double thresh, int n_warmup,
+                      int conserve_norm, const tdvp_heff2_term* terms, int nterms, int Dl, int d1, int d2, int Dr,
+                      tdvp_c128* theta_inout, int* niter) {
+  H_CHECK(h);
+  if (!terms || !theta_inout || nterms <= 0 || Dl <= 0 || d1 <= 0 || d2 <= 0 || Dr <= 0) { set_error(h, "krylov_expm2: bad argument"); return TDVP_ERR_ARG; }
+  return krylov_expm2_exec(h, kind, scale_re, scale_im, thresh, n_warmup, conserve_norm, terms, nterms, Dl, d1, d2, Dr,
+                           (c128*)theta_inout, niter);
 }
 
 int tdvp_keff_apply(tdvp_handle_t h, const tdvp_keff_term* terms, int nterms, int Dl, int Dr, const tdvp_c128* sigma,

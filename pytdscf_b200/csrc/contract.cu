@@ -11,6 +11,8 @@
 //   T2[a,i,t,s] = sum_cj W[c,i,j,t] T1[a,c,j,s]              GEMM (Dl*Dr) x (d*wr) x (wl*d), two-level rows
 //   out[a,i,r] += sum_ts T2[a,i,t,s] R[r,t,s]                GEMM (Dl*d) x Dr x (wr*Dr), B operand K-major
 // The term sum is folded into the last GEMM's epilogue (beta = 1), so no separate accumulation pass.
+#include <algorithm>
+
 #include "contract.cuh"
 
 namespace tdvp {
@@ -332,6 +334,173 @@ int heff_term_exec(Handle* h, const tdvp_heff_term& t, int Dl, int d, int Dr, co
 int heff_apply_exec(Handle* h, const tdvp_heff_term* terms, int nterms, int Dl, int d, int Dr, const c128* psi, c128* out) {
   if (nterms <= 0) { set_error(h, "heff_apply: no terms"); return TDVP_ERR_ARG; }
   for (int i = 0; i < nterms; ++i) TDVP_TRY(heff_term_exec(h, terms[i], Dl, d, Dr, psi, out, i > 0));
+  return 0;
+}
+
+// ---- two-site H_eff ----------------------------------------------------------------------------------------------
+// out[a,i,k,r] = coef * sum L[a,c,b] W1[c,i,j,t] W2[t,k,l,u] R[r,u,s] theta[b,j,l,s] as the one-site chain with
+// reinterpreted sizes (every operand keeps its natural layout):
+//   s1  T1[a,c,(j l s)]   = sum_b L[a,c,b] theta[b,(j l s)]           one-site s1 with d = d1 d2
+//   s2  T2[a,i,t,(l s)]   = sum_cj W1 T1                              one-site s2 with (Dl, wl, d1, wm, Dr' = d2 Dr)
+//   s3  T3[(a i),k,u,s]   = sum_tl W2 T2                              one-site s2 with (Dl' = Dl d1, wm, d2, wr, Dr)
+//   s4  out[(a i k), r]   = sum_us T3 R                               one-site s3 with rows Dl d1 d2
+// T1 / T2 / T3 ping-pong between two workspace buffers.
+namespace {
+
+size_t heff2_stage_elems(const tdvp_heff2_term& t, int Dl, int d1, int d2, int Dr) {
+  const size_t wl = t.L ? t.wl : 1, wr = t.R ? t.wr : 1, wm = t.wm > 0 ? t.wm : 1;
+  const size_t n = (size_t)Dl * d1 * d2 * Dr;
+  size_t e = n * wl;                       // T1
+  if (n * wm > e) e = n * wm;              // T2
+  if (n * wr > e) e = n * wr;              // T3
+  return e;
+}
+
+// stage 2 with a diagonal core over Dl rows in chunks the grid's z extent can address
+int stage2_diag_rows(Handle* h, const c128* T1, const c128* Wd, c128* T2, long long Dl, int wl, int d, int wr, int Dr,
+                     c128 alpha, c128 beta) {
+  const long long chunk = 65535;
+  for (long long a0 = 0; a0 < Dl; a0 += chunk) {
+    const int rows = (int)(Dl - a0 < chunk ? Dl - a0 : chunk);
+    TDVP_TRY(stage2_diag(h, T1 + a0 * wl * d * Dr, Wd, T2 + a0 * d * wr * Dr, rows, wl, d, wr, Dr, alpha, beta));
+  }
+  return 0;
+}
+
+// one W stage of the two-site chain: dst = alpha * W . cur + beta * dst on (rows, w_in, d, w_out, cols)
+int heff2_mid(Handle* h, const c128* W, const c128* Wp, int kind, const c128* cur, c128* dst, long long rows, int w_in,
+              int d, int w_out, int cols, c128 alpha, c128 beta, const char* tag) {
+  if (kind == TDVP_KIND_FULL) {
+    if (!Wp) {
+      c128* tmp = (c128*)ws_alloc(h, sizeof(c128) * (size_t)w_in * d * d * w_out);
+      if (!tmp) { set_error(h, "workspace exhausted (heff2 Wp)"); return TDVP_ERR_ARG; }
+      { ProfScope _ps(h->stream, "aux.permute_w_kernel"); permute_w_kernel<<<grid_for((long long)w_in * d * d * w_out, 128, 64), 128, 0, h->stream>>>(W, tmp, w_in, d, w_out, 0); }
+      TDVP_TRY(launch_check(h, "permute_w_kernel"));
+      Wp = tmp;
+    }
+    // GEMM rows are (row, col) pairs; the smallest tile (32 rows) puts them on gridDim.y, which stops at 65535
+    const long long chunk = std::max(1ll, (65535ll * 32) / cols);
+    for (long long a0 = 0; a0 < rows; a0 += chunk) {
+      const int nr = (int)(rows - a0 < chunk ? rows - a0 : chunk);
+      TDVP_TRY(stage2_full(h, cur + a0 * w_in * d * cols, Wp, dst + a0 * d * w_out * cols, nr, w_in, d, w_out, cols, alpha,
+                           beta, tag));
+    }
+    return 0;
+  }
+  return stage2_diag_rows(h, cur, W, dst, rows, w_in, d, w_out, cols, alpha, beta);
+}
+
+}  // namespace
+
+size_t heff2_ws_elems(const tdvp_heff2_term* terms, int nterms, int Dl, int d1, int d2, int Dr) {
+  size_t need = 0;
+  for (int i = 0; i < nterms; ++i) {
+    const tdvp_heff2_term& t = terms[i];
+    const size_t wl = t.wl > 0 ? t.wl : 1, wm = t.wm > 0 ? t.wm : 1, wr = t.wr > 0 ? t.wr : 1;
+    size_t e = 2 * heff2_stage_elems(t, Dl, d1, d2, Dr) + wl * d1 * d1 * wm + wm * d2 * d2 * wr + 64 * 4;
+    if (e > need) need = e;
+  }
+  return need;
+}
+
+int heff2_term_exec(Handle* h, const tdvp_heff2_term& t, int Dl, int d1, int d2, int Dr, const c128* theta, c128* out,
+                    bool accumulate) {
+  const c128 coef = {t.coef_re, t.coef_im};
+  const c128 one = {1.0, 0.0}, zero = {0.0, 0.0};
+  const c128 beta_out = accumulate ? one : zero;
+  const c128* L = reinterpret_cast<const c128*>(t.L);
+  const c128* W1 = reinterpret_cast<const c128*>(t.W1);
+  const c128* W2 = reinterpret_cast<const c128*>(t.W2);
+  const c128* R = reinterpret_cast<const c128*>(t.R);
+  const int wl = t.wl, wm = t.wm, wr = t.wr;
+  if (wl < 1 || wm < 1 || wr < 1) { set_error(h, "heff2 term: MPO bond dimension < 1"); return TDVP_ERR_SHAPE; }
+  if ((!L && wl != 1) || (!R && wr != 1)) { set_error(h, "heff2 term: an identity block requires an MPO bond dimension of 1"); return TDVP_ERR_SHAPE; }
+  if ((!W1 && (wl != 1 || wm != 1)) || (!W2 && (wm != 1 || wr != 1))) {
+    set_error(h, "heff2 term: an identity core requires MPO bond dimensions of 1 on both of its sides");
+    return TDVP_ERR_UNSUPPORTED;
+  }
+  if ((W1 && t.w1_kind != TDVP_KIND_DIAG && t.w1_kind != TDVP_KIND_FULL) || (W2 && t.w2_kind != TDVP_KIND_DIAG && t.w2_kind != TDVP_KIND_FULL)) {
+    set_error(h, "heff2 term: bad core kind");
+    return TDVP_ERR_ARG;
+  }
+  const size_t top = h->ws_top;
+  const long long N = (long long)Dl * d1 * d2 * Dr;
+  int l_id = (t.id_channels & 0xffff) - 1, r_id = ((t.id_channels >> 16) & 0xffff) - 1;
+  if (N < ID_CHANNEL_MIN_ELEMS || !L || wl < 2 || l_id >= wl) l_id = -1;
+  if (N < ID_CHANNEL_MIN_ELEMS || !R || wr < 2 || r_id >= wr) r_id = -1;
+  // algorithmic flops F_H2
+  double fl = 0.0;
+  const double n = (double)Dl * d1 * d2 * Dr;
+  if (L) fl += 8.0 * n * Dl * wl;
+  if (W1) fl += 8.0 * n * (t.w1_kind == TDVP_KIND_FULL ? d1 : 1) * wl * wm;
+  if (W2) fl += 8.0 * n * (t.w2_kind == TDVP_KIND_FULL ? d2 : 1) * wm * wr;
+  if (R) fl += 8.0 * n * Dr * wr;
+  h->heff_flops += fl;
+
+  const size_t cap = heff2_stage_elems(t, Dl, d1, d2, Dr);
+  c128* buf[2] = {nullptr, nullptr};
+  const int nstages = (L ? 1 : 0) + (W1 ? 1 : 0) + (W2 ? 1 : 0) + (R ? 1 : 0);
+  const bool any_stage = nstages > 0;
+  if (nstages >= 2) {   // every stage but the last writes an intermediate
+    buf[0] = (c128*)ws_alloc(h, sizeof(c128) * cap);
+    buf[1] = (c128*)ws_alloc(h, sizeof(c128) * cap);
+    if (!buf[0] || !buf[1]) { set_error(h, "workspace exhausted (heff2 T)"); return TDVP_ERR_ARG; }
+  }
+  auto next = [&](const c128* cur) { return cur == buf[0] ? buf[1] : buf[0]; };
+  const c128* cur = theta;
+  int rc = 0;
+  // ---- s1 ----
+  if (L) {
+    const bool last = !W1 && !W2 && !R;
+    c128* dst = last ? out : next(cur);
+    if (l_id >= 0 && !last) {
+      if ((rc = left_apply_skip(h, L, Dl, wl, l_id, cur, (long long)d1 * d2 * Dr, dst, "heff2.s1"))) return rc;
+    } else {
+      GemmDesc g = gemm_rowmajor(Dl * wl, d1 * d2 * Dr, Dl, L, Dl, false, false, cur, (long long)d1 * d2 * Dr, false, dst,
+                                 (long long)d1 * d2 * Dr, last ? coef : one, last ? beta_out : zero);
+      g.tag = "heff2.s1";
+      if ((rc = gemm(h, g))) return rc;
+    }
+    cur = dst;
+  }
+  // ---- s2: W1 on (Dl, wl, d1, wm, d2 Dr) ----
+  if (W1) {
+    const bool last = !W2 && !R;
+    c128* dst = last ? out : next(cur);
+    if ((rc = heff2_mid(h, W1, reinterpret_cast<const c128*>(t.W1p), t.w1_kind, cur, dst, Dl, wl, d1, wm, d2 * Dr,
+                        last ? coef : one, last ? beta_out : zero, "heff2.s2"))) return rc;
+    cur = dst;
+  }
+  // ---- s3: W2 on (Dl d1, wm, d2, wr, Dr) ----
+  if (W2) {
+    const bool last = !R;
+    c128* dst = last ? out : next(cur);
+    if ((rc = heff2_mid(h, W2, reinterpret_cast<const c128*>(t.W2p), t.w2_kind, cur, dst, (long long)Dl * d1, wm, d2, wr, Dr,
+                        last ? coef : one, last ? beta_out : zero, "heff2.s3"))) return rc;
+    cur = dst;
+  }
+  // ---- s4 ----
+  if (R) {
+    const long long rows = (long long)Dl * d1 * d2;
+    if (r_id >= 0 && cur != theta) {
+      if ((rc = right_apply_skip(h, cur, rows, Dr, wr, r_id, R, out, coef, beta_out, "heff2.s4"))) return rc;
+    } else {
+      GemmDesc g = gemm_rowmajor((int)rows, Dr, wr * Dr, cur, (long long)wr * Dr, false, false, R, (long long)wr * Dr, true,
+                                 out, Dr, coef, beta_out);
+      g.tag = "heff2.s4";
+      if ((rc = gemm(h, g))) return rc;
+    }
+  } else if (!any_stage) {
+    if ((rc = axpby(h, theta, out, N, coef, beta_out))) return rc;
+  }
+  h->ws_top = top;
+  return 0;
+}
+
+int heff2_apply_exec(Handle* h, const tdvp_heff2_term* terms, int nterms, int Dl, int d1, int d2, int Dr, const c128* theta,
+                     c128* out) {
+  if (nterms <= 0) { set_error(h, "heff2_apply: no terms"); return TDVP_ERR_ARG; }
+  for (int i = 0; i < nterms; ++i) TDVP_TRY(heff2_term_exec(h, terms[i], Dl, d1, d2, Dr, theta, out, i > 0));
   return 0;
 }
 

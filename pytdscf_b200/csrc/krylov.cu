@@ -609,14 +609,14 @@ int inner_exec(Handle* h, long long n, const c128* bra, const c128* ket, int con
   return 0;
 }
 
-int krylov_expm_exec(Handle* h, int kind, double scale_re, double scale_im, double thresh, int n_warmup,
-                     int conserve_norm, const tdvp_heff_term* hterms, const tdvp_keff_term* kterms, int nterms,
-                     int Dl, int d, int Dr, c128* psi, int* niter) {
-  if ((hterms == nullptr) == (kterms == nullptr)) { set_error(h, "krylov_expm: pass exactly one of hterms / kterms"); return TDVP_ERR_ARG; }
-  if (kind != TDVP_KRYLOV_LANCZOS_REF && kind != TDVP_KRYLOV_ARNOLDI) { set_error(h, "krylov_expm: bad kind"); return TDVP_ERR_ARG; }
-  const bool isH = hterms != nullptr;
-  const long long N = isH ? (long long)Dl * d * Dr : (long long)Dl * Dr;
-  if (N <= 0) { set_error(h, "krylov_expm: empty vector"); return TDVP_ERR_SHAPE; }
+namespace {
+
+// exp(scale * Op) psi for an operator given as `apply(x, y)`: y = Op x on vectors of N elements; `contr` = workspace
+// elements the operator needs per application.  `checked`: report a workspace the device cannot hold as
+// TDVP_ERR_NO_MEMORY (the two-site solve, whose basis can outgrow the device).
+template <class Apply>
+int krylov_expm_core(Handle* h, int kind, double scale_re, double scale_im, double thresh, int n_warmup, int conserve_norm,
+                     long long N, size_t contr, bool checked, Apply&& apply, c128* psi, int* niter) {
   // The reference sizes the Krylov space (cap, warm-up bound, "space exhausted" test) by the tensor it was GIVEN; with
   // adaptive bond growth that tensor is smaller than the zero-extended vector the recurrence runs on
   // (_integrator.py:178-186, 524, 570): tdvp_set_krylov_size passes that size for the next solve.
@@ -628,9 +628,9 @@ int krylov_expm_exec(Handle* h, int kind, double scale_re, double scale_im, doub
   if (n_warm < 0) n_warm = 0;
 
   // ---- workspace: V[(ndim+1) x N], y, prev, + contraction scratch ----
-  const size_t contr = isH ? heff_ws_elems(hterms, nterms, Dl, d, Dr) : keff_ws_elems(kterms, nterms, Dl, Dr);
   const size_t need = sizeof(c128) * ((size_t)(ndim + 3) * N + contr) + 256 * 16;
-  TDVP_TRY(ws_reserve(h, need));
+  if (checked) TDVP_TRY(ws_reserve_checked(h, need, "krylov_expm2 (Krylov basis)"));
+  else TDVP_TRY(ws_reserve(h, need));
   c128* V = (c128*)ws_alloc(h, sizeof(c128) * (size_t)(ndim + 1) * N);
   c128* ybuf[2] = {(c128*)ws_alloc(h, sizeof(c128) * N), (c128*)ws_alloc(h, sizeof(c128) * N)};
   if (!V || !ybuf[0] || !ybuf[1]) { set_error(h, "krylov_expm: workspace"); return TDVP_ERR_ARG; }
@@ -641,7 +641,7 @@ int krylov_expm_exec(Handle* h, int kind, double scale_re, double scale_im, doub
 
   auto matvec = [&](const c128* x, c128* y) -> int {
     ++h->krylov_matvecs;
-    return isH ? heff_apply_exec(h, hterms, nterms, Dl, d, Dr, x, y) : keff_apply_exec(h, kterms, nterms, Dl, Dr, x, y);
+    return apply(x, y);
   };
 
   // ---- v0 ----
@@ -776,6 +776,37 @@ int krylov_expm_exec(Handle* h, int kind, double scale_re, double scale_im, doub
   set_error(h, kind == TDVP_KRYLOV_ARNOLDI ? "Short Iterative Arnoldi is not converged in 20 basis"
                                            : "Short Iterative Lanczos is not converged. Try shorter time interval.");
   return TDVP_ERR_NOT_CONVERGED;
+}
+
+}  // namespace
+
+int krylov_expm_exec(Handle* h, int kind, double scale_re, double scale_im, double thresh, int n_warmup,
+                     int conserve_norm, const tdvp_heff_term* hterms, const tdvp_keff_term* kterms, int nterms,
+                     int Dl, int d, int Dr, c128* psi, int* niter) {
+  if ((hterms == nullptr) == (kterms == nullptr)) { set_error(h, "krylov_expm: pass exactly one of hterms / kterms"); return TDVP_ERR_ARG; }
+  if (kind != TDVP_KRYLOV_LANCZOS_REF && kind != TDVP_KRYLOV_ARNOLDI) { set_error(h, "krylov_expm: bad kind"); return TDVP_ERR_ARG; }
+  const bool isH = hterms != nullptr;
+  const long long N = isH ? (long long)Dl * d * Dr : (long long)Dl * Dr;
+  if (N <= 0) { set_error(h, "krylov_expm: empty vector"); return TDVP_ERR_SHAPE; }
+  const size_t contr = isH ? heff_ws_elems(hterms, nterms, Dl, d, Dr) : keff_ws_elems(kterms, nterms, Dl, Dr);
+  return krylov_expm_core(h, kind, scale_re, scale_im, thresh, n_warmup, conserve_norm, N, contr, false,
+                          [&](const c128* x, c128* y) {
+                            return isH ? heff_apply_exec(h, hterms, nterms, Dl, d, Dr, x, y)
+                                       : keff_apply_exec(h, kterms, nterms, Dl, Dr, x, y);
+                          },
+                          psi, niter);
+}
+
+// Two-site operator: theta(Dl, d1, d2, Dr), the same solver on the heff2 chain.
+int krylov_expm2_exec(Handle* h, int kind, double scale_re, double scale_im, double thresh, int n_warmup,
+                      int conserve_norm, const tdvp_heff2_term* terms, int nterms, int Dl, int d1, int d2, int Dr, c128* theta,
+                      int* niter) {
+  if (kind != TDVP_KRYLOV_LANCZOS_REF && kind != TDVP_KRYLOV_ARNOLDI) { set_error(h, "krylov_expm2: bad kind"); return TDVP_ERR_ARG; }
+  const long long N = (long long)Dl * d1 * d2 * Dr;
+  const size_t contr = heff2_ws_elems(terms, nterms, Dl, d1, d2, Dr);
+  return krylov_expm_core(h, kind, scale_re, scale_im, thresh, n_warmup, conserve_norm, N, contr, true,
+                          [&](const c128* x, c128* y) { return heff2_apply_exec(h, terms, nterms, Dl, d1, d2, Dr, x, y); },
+                          theta, niter);
 }
 
 // Lowest (root = 0) / highest eigenvector of the effective Hamiltonian by textbook Lanczos -- the site solve of

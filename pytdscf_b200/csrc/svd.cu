@@ -434,6 +434,25 @@ __global__ void k_pinv_diag(const c128* __restrict__ X, int n, double cut, c128*
   }
 }
 
+// out[i, j] = f * (trans ? conj(src[j * ld + i]) : src[i * ld + j]) on an (rows x cols) row-major output, with
+// f = scale[i] (by_col == 0), scale[j] (by_col == 1) or 1 (scale == nullptr).  Forms the factors of tdvp_split2.
+__global__ void k_split_factor(const c128* __restrict__ src, long long ld, int trans, long long rows, int cols,
+                               const double* __restrict__ scale, int by_col, c128* __restrict__ out) {
+  const long long tot = rows * cols;
+  for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < tot; e += (long long)gridDim.x * blockDim.x) {
+    const long long i = e / cols;
+    const int j = (int)(e % cols);
+    c128 v = trans ? src[(long long)j * ld + i] : src[i * ld + j];
+    if (trans) v.y = -v.y;
+    if (scale) {
+      const double f = scale[by_col ? j : i];
+      v.x *= f;
+      v.y *= f;
+    }
+    out[e] = v;
+  }
+}
+
 int ls(Handle* h, const char* what) {
   count_launch();
   cudaError_t e = cudaGetLastError();
@@ -622,6 +641,75 @@ int tdvp_svd(tdvp_handle_t hh, int m, int n, const tdvp_c128* A, tdvp_c128* U, d
   h->err.clear();
   if (!A || !U || !s_host || !Vh || m <= 0 || n <= 0 || m < n) { set_error(h, "svd: bad argument (needs m >= n)"); return TDVP_ERR_ARG; }
   return svd_exec(h, m, n, (const c128*)A, (c128*)U, (c128*)Vh, s_host);
+}
+
+int tdvp_split2(tdvp_handle_t hh, int direction, int Dl, int d1, int d2, int Dr, const tdvp_c128* theta, double p,
+                int Dcap, int conserve_norm, tdvp_c128* left, tdvp_c128* right, double* s_host, int* rank) {
+  Handle* h = reinterpret_cast<Handle*>(hh);
+  if (!h) return TDVP_ERR_ARG;
+  h->err.clear();
+  if (!theta || !left || !right || !s_host || !rank || Dl <= 0 || d1 <= 0 || d2 <= 0 || Dr <= 0 || Dcap <= 0 ||
+      (direction != TDVP_GAUGE_A && direction != TDVP_GAUGE_B) || !(p >= 0.0 && p < 1.0)) {
+    set_error(h, "split2: bad argument");
+    return TDVP_ERR_ARG;
+  }
+  const long long m = (long long)Dl * d1, n = (long long)d2 * Dr;
+  if (m > INT32_MAX || n > INT32_MAX) { set_error(h, "split2: matricisation too large"); return TDVP_ERR_SHAPE; }
+  // SVD of the tall one of theta (m x n) and theta^H (n x m): A(M x K) = Ua diag(s) Vha, K = min(m, n)
+  const bool wide = m < n;
+  const int M = (int)(wide ? n : m), K = (int)(wide ? m : n);
+  const size_t bytes = svd_ws_bytes(M, K) + align256(sizeof(c128) * (size_t)M * K) * (wide ? 2 : 1) +
+                       align256(sizeof(c128) * (size_t)K * K) + align256(sizeof(double) * K) + 4096;
+  TDVP_TRY(ws_reserve_checked(h, bytes, "split2"));
+  c128* A = nullptr;
+  if (wide) {
+    A = (c128*)ws_alloc(h, sizeof(c128) * (size_t)M * K);
+    if (!A) { set_error(h, "split2: workspace"); return TDVP_ERR_ARG; }
+    { ProfScope _ps(h->stream, "svd.k_split_factor"); k_split_factor<<<148 * 2, 256, 0, h->stream>>>((const c128*)theta, n, 1, M, K, nullptr, 0, A); }
+    TDVP_TRY(ls(h, "k_split_factor"));
+  }
+  c128* Ua = (c128*)ws_alloc(h, sizeof(c128) * (size_t)M * K);
+  c128* Vha = (c128*)ws_alloc(h, sizeof(c128) * (size_t)K * K);
+  double* dscale = (double*)ws_alloc(h, sizeof(double) * K);
+  if (!Ua || !Vha || !dscale) { set_error(h, "split2: workspace"); return TDVP_ERR_ARG; }
+  std::vector<double> s(K);
+  TDVP_TRY(svd_exec(h, M, K, wide ? A : (const c128*)theta, Ua, Vha, s.data(), false));
+  // rank: cumulative singular-VALUE weight, as tdvp_svd_truncate; then the static cap
+  double total = 0.0;
+  for (int i = 0; i < K; ++i) total += s[i];
+  int rp = K;
+  if (total > 0.0) {
+    double acc = 0.0;
+    for (int i = 0; i < K; ++i) { acc += s[i]; if (acc / total >= 1.0 - p) { rp = i + 1; break; } }
+  }
+  int r = rp < Dcap ? rp : Dcap;
+  if (r > K) r = K;
+  if (r < 1) r = 1;
+  double f = 1.0;
+  if (conserve_norm) {
+    double all = 0.0, kept = 0.0;
+    for (int i = 0; i < K; ++i) all += s[i] * s[i];
+    for (int i = 0; i < r; ++i) kept += s[i] * s[i];
+    if (kept > 0.0) f = std::sqrt(all) / std::sqrt(kept);
+  }
+  std::vector<double> sk(r);
+  for (int i = 0; i < r; ++i) sk[i] = s[i] * f;
+  TDVP_CUDA(h, cudaMemcpyAsync(dscale, sk.data(), sizeof(double) * r, cudaMemcpyHostToDevice, h->stream));
+  // theta = U diag(s) Vh with U = Ua, Vh = Vha (tall) or U = Vha^H, Vh = Ua^H (wide)
+  const bool s_left = direction == TDVP_GAUGE_B;
+  cudaStream_t st = h->stream;
+  { ProfScope _ps(st, "svd.k_split_factor");
+    if (!wide) k_split_factor<<<148 * 2, 256, 0, st>>>(Ua, K, 0, m, r, s_left ? dscale : nullptr, 1, (c128*)left);
+    else k_split_factor<<<148 * 2, 256, 0, st>>>(Vha, K, 1, m, r, s_left ? dscale : nullptr, 1, (c128*)left); }
+  TDVP_TRY(ls(h, "k_split_factor"));
+  { ProfScope _ps(st, "svd.k_split_factor");
+    if (!wide) k_split_factor<<<148 * 2, 256, 0, st>>>(Vha, K, 0, r, (int)n, s_left ? nullptr : dscale, 0, (c128*)right);
+    else k_split_factor<<<148 * 2, 256, 0, st>>>(Ua, K, 1, r, (int)n, s_left ? nullptr : dscale, 0, (c128*)right); }
+  TDVP_TRY(ls(h, "k_split_factor"));
+  TDVP_CUDA(h, cudaStreamSynchronize(st));   // sk is a host temporary of the copy above
+  for (int i = 0; i < K; ++i) s_host[i] = s[i];
+  *rank = r;
+  return 0;
 }
 
 int tdvp_pinv(tdvp_handle_t hh, int m, int n, const tdvp_c128* X, double rcond, tdvp_c128* out) {

@@ -274,8 +274,26 @@ class Simulator:
                   adaptive: bool = False, adaptive_Dmax: int = 20, adaptive_dD: int = 5,
                   adaptive_p_proj: float = 1.0e-04, adaptive_p_svd: float = 1.0e-07, integrator: str = "lanczos",
                   display_time_unit: str = "fs", conserve_norm: bool = True, write_files: bool = True,
-                  record_trace: bool = False):
-        """Real-time propagation; returns ``(energy, wf)`` like the reference (energy of the last evaluated step)."""
+                  record_trace: bool = False, two_site: bool = False, two_site_p_svd: float = 1.0e-07):
+        """Real-time propagation; returns ``(energy, wf)`` like the reference (energy of the last evaluated step).
+
+        ``two_site=True``: two-site TDVP -- every pair of neighbouring sites is propagated together and split again by a
+        truncated SVD, so the bond dimensions follow the state (from a Hartree product up to the model's ``bond_dim``):
+        the smallest rank whose cumulative singular-value sum reaches ``1 - two_site_p_svd`` of the total is kept.  Bond
+        dimensions are written to ``bonddim.dat`` and ``history``.  Not combined with ``adaptive``, site-parallel runs,
+        gates or Kraus maps."""
+        if two_site:
+            if adaptive:
+                raise NotImplementedError("two_site=True and adaptive=True are alternative bond-growth schemes; pick one")
+            if parallel_split_indices is not None:
+                raise NotImplementedError("two-site TDVP is not implemented for site-parallel runs")
+            if self.model.one_gate_to_apply is not None or self.model.kraus_op is not None:
+                raise NotImplementedError("two-site TDVP applies no gates or Kraus maps between its half sweeps")
+            if self.model.get_ndof() < 2:
+                raise ValueError("two-site TDVP needs a chain of at least two sites")
+            if not 0.0 <= two_site_p_svd < 1.0:
+                raise ValueError(f"two_site_p_svd must lie in [0, 1), got {two_site_p_svd}")
+        self._two_site = (bool(two_site), float(two_site_p_svd))
         self._rd = None
         if reduced_density is not None:
             keys, rd_step = reduced_density
@@ -312,6 +330,10 @@ class Simulator:
                         verbose=self.verbose, space=self.model.space, integrator=integrator, conserve_norm=conserve_norm,
                         display_time_unit=display_time_unit, adaptive=adaptive, p_svd=p_svd, Dmax=int(adaptive_params[0]),
                         dD=int(adaptive_params[1]), p_proj=float(adaptive_params[2]))
+        if not relax and getattr(self, "_two_site", (False, 0.0))[0]:
+            cfg.two_site, cfg.two_site_p_svd = True, self._two_site[1]
+            cfg.bond_dim = int(self.model.m_aux_max or 0)
+        self._two_site = (False, 0.0)
         self.cfg = cfg
         split = getattr(self, "_split", None) if not relax else None
         if split is not None:
@@ -348,7 +370,7 @@ class Simulator:
                 rec["pops"] = wf.pop_states()
             if observables and istep % observables_per_step == 0:
                 rec["expectations"] = {k: wf.expectation(op) for k, op in self.model.observables.items()}
-            if cfg.adaptive:
+            if cfg.adaptive or cfg.two_site:
                 rec["bonddim"] = wf.bonddim()
             rd = getattr(self, "_rd", None)
             if rd is not None and not relax and istep % rd[2] == 0:
@@ -379,9 +401,12 @@ class Simulator:
     def relax(self, stepsize: float = 0.1, maxstep: int = 20, improved: bool = True, restart: bool = False,
               savefile_ext: str = "_gs", loadfile_ext: str = "", backup_interval: int = 10, norm: bool = True,
               populations: bool = True, observables: bool = False, integrator: str = "lanczos",
-              display_time_unit: str = "fs", write_files: bool = True, record_trace: bool = False):
+              display_time_unit: str = "fs", write_files: bool = True, record_trace: bool = False,
+              two_site: bool = False):
         """Ground-state relaxation (reference ``simulator_cls.py:95-158``): improved relaxation (per-site Lanczos
-        eigen-solve, default) or imaginary-time propagation.  Returns ``(energy, wf)``."""
+        eigen-solve, default) or imaginary-time propagation.  Returns ``(energy, wf)``.  One-site only."""
+        if two_site:
+            raise NotImplementedError("two-site relaxation is not implemented; relax runs the one-site scheme")
         return self._run(stepsize, maxstep, "improved" if improved else True, restart, savefile_ext, loadfile_ext,
                          backup_interval, autocorr=False, energy=True, norm=norm, populations=populations,
                          observables=observables, thresh_sil=1.0e-09, integrator=integrator,
@@ -389,11 +414,13 @@ class Simulator:
                          record_trace=record_trace, suffix="_relax")
 
     def operate(self, maxstep: int = 10, restart: bool = False, savefile_ext: str = "_operate", loadfile_ext: str = "_gs",
-                verbose: int = 2, write_files: bool = True):
+                verbose: int = 2, write_files: bool = True, two_site: bool = False):
         """Apply the model's ``hamiltonian`` entry -- in this mode an operator such as a dipole MPO -- to the wavefunction
         (reference ``Simulator.operate``, simulator_cls.py:286-330, 356-361): |Psi'> = O|Psi> / |O|Psi>|.  Returns
         ``(|O|Psi>|, wf)`` and writes ``wf_<jobname><savefile_ext>.pkl``, from which ``propagate(restart=True, loadfile_ext=
         savefile_ext)`` continues -- the relax -> operate -> propagate workflow of the reference's spectra notebooks."""
+        if two_site:
+            raise NotImplementedError("operate fits O|Psi> with one-site sweeps; there is no two-site variant")
         if self.model.space != "hilbert":
             raise NotImplementedError("operate is implemented for Hilbert-space MPS")
         wf = self.get_initial_wavefunction(restart, loadfile_ext)
@@ -418,7 +445,7 @@ class Simulator:
         os.makedirs(cfg.jobname, exist_ok=True)
         return {name: _DatFile(os.path.join(cfg.jobname, fn)) for name, fn in
                 (("main", "main.log"), ("auto", "autocorr.dat"), ("pop", "populations.dat"), ("exp", "expectations.dat"))
-                + ((("bond", "bonddim.dat"),) if cfg.adaptive else ())}
+                + ((("bond", "bonddim.dat"),) if cfg.adaptive or cfg.two_site else ())}
 
     def _export(self, files: dict, cfg: RunConfig, rec: dict, elapsed: float):
         unit = cfg.display_time_unit
@@ -433,7 +460,7 @@ class Simulator:
             if first:
                 files["pop"].write(f"# time [{unit}]\t" + "\t".join(f"pop_{i}".ljust(11) for i in range(len(rec["pops"]))))
             files["pop"].write(f"{t:6.9f}\t" + "".join(f"{p:6.9f}\t" for p in rec["pops"]))
-        if "bonddim" in rec and "bond" in files:     # adaptive runs: properties.py:344-356
+        if "bonddim" in rec and "bond" in files:     # adaptive and two-site runs: properties.py:344-356
             if first:
                 files["bond"].write(f"# time [{unit}]\t" + "\t".join(f"{i}" for i in range(len(rec["bonddim"]))))
             files["bond"].write(f"{t:6.9f}\t" + "".join(f"{b}\t" for b in rec["bonddim"]))
