@@ -166,7 +166,9 @@ int tdvp_overlap_site(tdvp_handle_t h, int Dlb, int Dlk, int d, int Drb, int Drk
                       const tdvp_c128* ket, const tdvp_c128* block, int conj_bra, tdvp_c128* out);
 
 /* ---- plain GEMM (exposed for tests / bench) ------------------------------------------------------ */
-/* C(M,N) = alpha * op(A) . op(B) + beta * C, row-major; transX: 0 = N, 1 = T, 2 = C (conjugate transpose). */
+/* C(M,N) = alpha * op(A) . op(B) + beta * C, row-major; transX: 0 = N, 1 = T, 2 = C (conjugate transpose).
+ * K = 0 gives C = beta * C (beta = 0: zeros, C is not read).  TDVP_ERR_ARG when lda, ldb or ldc is smaller than the
+ * row length of its matrix as stored (A: K, or M when transposed; B: N, or K when transposed; C: N). */
 int tdvp_zgemm(tdvp_handle_t h, int transA, int transB, int M, int N, int K, double alpha_re,
                double alpha_im, const tdvp_c128* A, int lda, const tdvp_c128* B, int ldb, double beta_re,
                double beta_im, tdvp_c128* C, int ldc);

@@ -314,6 +314,11 @@ int tdvp_zgemm(tdvp_handle_t h, int transA, int transB, int M, int N, int K, dou
     set_error(h, "zgemm: bad argument");
     return TDVP_ERR_ARG;
   }
+  // a leading dimension shorter than its matrix's rows would make the kernels address past the end of the buffer
+  if (lda < (transA ? M : K) || ldb < (transB ? K : N) || ldc < N) {
+    set_error(h, "zgemm: a leading dimension is smaller than its row length");
+    return TDVP_ERR_ARG;
+  }
   GemmDesc g = gemm_rowmajor(M, N, K, (const c128*)A, lda, transA != 0, transA == 2, (const c128*)B, ldb, transB != 0,
                              (c128*)C, ldc, c128{alpha_re, alpha_im}, c128{beta_re, beta_im});
   g.b_conj = transB == 2 ? 1 : 0;

@@ -237,12 +237,13 @@ __global__ void __launch_bounds__(C::THREADS, C::THREADS == 256 ? 1 : 4) zgemm_d
   const int wm = warp % C::WMW, wn = warp / C::WMW;
   // Grouped rasterisation: consecutive CTAs walk 16 M-tiles for one N-tile before moving to the next N-tile, so a wave of
   // 148 CTAs works on a 16 x ~9 block of tiles (A rows stay in L2 for the whole group, B columns are read once per
-  // group) instead of ~2 full tile rows that stream all of B through L2 every wave.
+  // group) instead of ~2 full tile rows that stream all of B through L2 every wave.  blockIdx.x enumerates all tiles:
+  // gridDim.y stops at 65535, which would cap M at 65535 tiles.
   int tile_m, tile_n;
   {
     constexpr int GROUP_M = 16;
-    const int npm = gridDim.y, npn = gridDim.x;
-    const int pid = blockIdx.y * npn + blockIdx.x;
+    const int npm = (d.M + BM - 1) / BM, npn = (d.N + BN - 1) / BN;
+    const int pid = blockIdx.x;
     const int in_group = GROUP_M * npn;
     const int first_m = (pid / in_group) * GROUP_M;
     const int gsz = (npm - first_m) < GROUP_M ? (npm - first_m) : GROUP_M;
@@ -421,7 +422,7 @@ cudaError_t configure_cfg() {
 
 template <typename C>
 cudaError_t launch_cfg(const GemmDesc& d, cudaStream_t stream) {
-  dim3 grid((d.N + C::BN - 1) / C::BN, (d.M + C::BM - 1) / C::BM, d.batch * d.splitk);
+  dim3 grid(((d.N + C::BN - 1) / C::BN) * ((d.M + C::BM - 1) / C::BM), 1, d.batch * d.splitk);
   const bool ak = (d.a_k == 1), bk = (d.b_k == 1);
   ProfScope scope(stream, d.tag, 8.0 * (double)d.M * (double)d.N * (double)d.K * (double)d.batch, true);
   if (d.cluster_sk) {
@@ -494,8 +495,35 @@ cudaError_t zgemm_configure_device(GemmCtx& ctx) {
   return configure_cfg<TinyCfg>();
 }
 
+namespace {
+// k_splitk_reduce over S partial products at P on the C of `d` (S = 0: C = beta C, no partial is read)
+cudaError_t launch_reduce(const c128* P, int S, const GemmDesc& d, cudaStream_t stream) {
+  const long long tot = (long long)d.M * d.N;
+  int blocks = (int)((tot + 255) / 256);
+  if (blocks > 148 * 8) blocks = 148 * 8;
+  {
+    ProfScope scope(stream, "aux.k_splitk_reduce");
+    k_splitk_reduce<<<blocks, 256, 0, stream>>>(P, S, d.M, d.N, tot, d);
+  }
+  count_launch();
+  return cudaGetLastError();
+}
+}  // namespace
+
 cudaError_t zgemm_auto(const GemmDesc& d, const GemmCtx& ctx) {
   if (d.M <= 0 || d.N <= 0 || d.batch <= 0) return cudaSuccess;
+  if (d.K <= 0) {
+    // BLAS semantics of an empty sum: C = beta C through C's own addressing (beta = 0 writes zeros without reading C);
+    // alpha = 0 so that an infinite alpha does not turn the empty sum into NaN
+    GemmDesc g = d;
+    g.alpha = {0.0, 0.0};
+    for (int b = 0; b < d.batch; ++b) {
+      g.C = d.C + (long long)b * d.c_batch;
+      const cudaError_t e = launch_reduce(nullptr, 0, g, ctx.stream);
+      if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
+  }
   const GemmPlan pl = plan_gemm(d, ctx);
   GemmDesc g = d;
   g.c_stream = pl.c_stream;
@@ -516,15 +544,7 @@ cudaError_t zgemm_auto(const GemmDesc& d, const GemmCtx& ctx) {
   const bool tma = pl.kernel == GEMM_TMA_WIDE || pl.kernel == GEMM_TMA_TALL;
   cudaError_t e = tma ? zgemm_tma_launch(g, pl, ctx) : zgemm_dmma_launch(pl.kernel, g, ctx.stream);
   if (e != cudaSuccess || pl.reduce != REDUCE_SCRATCH) return e;
-  const long long tot = (long long)d.M * d.N;
-  int blocks = (int)((tot + 255) / 256);
-  if (blocks > 148 * 8) blocks = 148 * 8;
-  {
-    ProfScope scope(ctx.stream, "aux.k_splitk_reduce");
-    k_splitk_reduce<<<blocks, 256, 0, ctx.stream>>>(ctx.scratch, pl.S, d.M, d.N, (long long)d.M * d.N, d);
-  }
-  count_launch();
-  return cudaGetLastError();
+  return launch_reduce(ctx.scratch, pl.S, d, ctx.stream);
 }
 
 }  // namespace tdvp

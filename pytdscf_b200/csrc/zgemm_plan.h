@@ -220,9 +220,12 @@ inline void plan_streamk(GemmPlan& pl, long long total, int KT, const GemmCtx& c
   }
 }
 
-// Plan of `d` (M, N, batch > 0; its split-K fields at their defaults) under the handle's context.
+// Plan of `d` (M, N, batch > 0, K >= 0; its split-K fields at their defaults) under the handle's context.
 inline GemmPlan plan_gemm(const GemmDesc& d, const GemmCtx& ctx) {
   GemmPlan pl;
+  // K = 0: there is nothing to multiply (zgemm_auto computes C = beta C without a GEMM kernel); the default plan, one
+  // split of zero k-tiles, keeps the cost model below from dividing by a zero chunk
+  if (d.K <= 0) return pl;
   // ---- can tensor maps describe both operands?  N <= 32 with enough rows to fill the machine with 256-row tiles: tall
   const bool tall = d.N <= 32 && d.M >= 256 * 148;
   const int tbm = tall ? TallCfg::BM : WideCfg::BM, tbn = tall ? TallCfg::BN : WideCfg::BN;

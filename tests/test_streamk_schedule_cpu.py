@@ -210,3 +210,15 @@ def test_planned_schedule_covers_the_work_once(shim, M, N, K, layout, force_cfg,
             count += k1 - k0
     per_split = [-(-min(chunk, K - s * chunk) // 16) for s in range(S)] if S > 1 else [KT]
     assert count == len(seen) == p["tiles_m"] * p["tiles_n"] * sum(per_split)   # every (tile, split, k-tile) exactly once
+
+
+@pytest.mark.parametrize("M,N,layout", [(7, 5, "NN"), (4096, 4096, "NT"), (37888, 16, "2r"), (1024, 32, "TN")])
+@pytest.mark.parametrize("force_cfg,force_splitk", [(0, 0), (1, 4), (3, 3), (2, 16), (4, 0), (5, 1)])
+def test_plan_k0(shim, M, N, layout, force_cfg, force_splitk):
+    """K = 0 (an empty sum: zgemm_auto computes C = beta C without a GEMM kernel) plans one split and no reduction instead
+    of dividing by a zero k-chunk."""
+    a_in, a1, a0, ak, b_in, b1, b0, bk = operands(layout, M, N, 0, 64)
+    p = plan(shim, (M, N, 0, 1, A_ADDR, a_in, a1, a0, ak, B_ADDR, b_in, b1, b0, bk), force_cfg=force_cfg,
+             force_splitk=force_splitk)
+    assert (p["S"], p["reduce"], p["streamk"]) == (1, REDUCE_NONE, 0), p
+    assert p["kernel"] not in (GEMM_TMA_WIDE, GEMM_TMA_TALL), p
